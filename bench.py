@@ -22,6 +22,10 @@ roofline : FP32 issue roofline (SURVEY.md §8d): algorithmic lane-ops of the fra
 Outside the timed region the line also carries: `sustained` (>= 2 s of back-to-back frames),
 `cold_first_frame_ms`, `ms_per_step_with_tile_seed`, `extra_workloads` (BASELINE configs C2, C3, C5
 and the C4 batch at this N) and `cpu_baseline` (the reference's CPU renderer on this box's cores).
+
+--dump-outputs DIR writes the frame the last timed step computed (float32 RGBA, height x width x 4) as
+DIR/frame.npy; the inputs are fixed, so two builds can be compared output for output.  (Under the
+MCSKIN_BENCH_SPLIT tuning aid the step renders one part of the frame, and only that part is filled.)
 """
 from __future__ import annotations
 
@@ -40,6 +44,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 WORKLOAD = "headline_1080p_16spp_4b"
 # ncu counters of one frame of the committed code (tools/ncu_frame_counters.py): warp instructions and DRAM bytes
@@ -155,6 +160,12 @@ def dist_env():
     return int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
 
 
+def dump_frame(out_dir: str, frame: np.ndarray):
+    """DIR/frame.npy: the float32 RGBA frame of the last timed step (1080p: 33 MB)."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "frame.npy"), np.ascontiguousarray(frame, dtype=np.float32))
+
+
 # ------------------------------------------------------------------------- reference arm
 def cpu_reference_run(entry_name: str, steps: int, warmup: int):
     """Times the reference's own CPU renderer (oracle/_ref when it was built, else the C port)."""
@@ -177,12 +188,12 @@ def cpu_reference_run(entry_name: str, steps: int, warmup: int):
     times = []
     for i in range(warmup + steps):
         t0 = time.perf_counter()
-        runner.render(scene, cfg)
+        image = runner.render(scene, cfg)
         dt = time.perf_counter() - t0
         if i >= warmup:
             times.append(dt)
     sec = sum(times) / len(times)
-    return {"value": entry["unique_rays"] / sec / 1e6, "unit": "Mrays/s", "cores": cores, "kind": kind,
+    return {"value": entry["unique_rays"] / sec / 1e6, "unit": "Mrays/s", "cores": cores, "kind": kind, "image": image,
             "sample": f"{entry_name}: the full {entry['config']['width']}x{entry['config']['height']} frame at "
                       f"{entry['config']['samples_per_pixel']} spp ({entry['unique_rays']} unique rays) through "
                       f"TileRenderer::render, threadCount=0, mean of {len(times)} run(s) after {warmup} warm-up run(s)",
@@ -195,6 +206,8 @@ def run_reference_arm(args):
         return
     # every step is the whole headline frame (16 spp): the same config as the own arm's step
     res = cpu_reference_run(WORKLOAD, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_frame(args.dump_outputs, res["image"])
     counts = load_counts()
     line = {
         "impl": "reference", "metric": "Mrays/s", "value": res["value"], "unit": "Mrays/s", "n_gpus": args.gpus,
@@ -423,6 +436,11 @@ def run_own_arm(args):
     n_active = st["n_active_pixels"]
     if job.peer is not None:
         job.peer.check_timeout()
+    if args.dump_outputs:  # before the legs below render into the same frame again
+        if world > 1:
+            dist.barrier()  # the peers' stores into the root's frame (time_steps ends with one more) are complete
+        if rank == 0:
+            dump_frame(args.dump_outputs, job.frame.cpu().numpy())
 
     # ---- pass breakdown, outside the timed region: the same frame on ONE stream with direct launches
     # (the timed frames interleave several lanes inside a CUDA graph, where pass times overlap)
@@ -708,7 +726,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra_workloads leg")
     ap.add_argument("--kernel-only", action="store_true", help="tuning runs: only the timed frames and the pass breakdown")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frame of the last timed step to DIR/frame.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference_arm(args)

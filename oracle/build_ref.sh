@@ -1,20 +1,30 @@
 #!/usr/bin/env bash
 # build_ref.sh — TEST INFRASTRUCTURE.  Compiles the UNMODIFIED reference core from
-# where it lies (/root/reference, read-only) plus oracle/ref_shim.cpp into
-# oracle/_ref/libmcskin_ref.so.  Only outputs land under oracle/_ref/ (git-ignored,
-# NOT gpurun-ignored: the .so travels to the GPU box, the reference sources do not).
+# a checkout of it (read-only; not part of this repository): the one
+# MCSKIN_REFERENCE_DIR names, else `reference` beside this repository.  Adds
+# oracle/ref_shim.cpp and links oracle/_ref/libmcskin_ref.so.  Only outputs land
+# under oracle/_ref/ (git-ignored).
 #
 # Flags = the reference's Release configuration (scripts/package.sh:57 ->
 # CMAKE_BUILD_TYPE=Release -> -O3 -DNDEBUG, C++17, no -march, no fast-math), i.e.
 # x86-64 baseline: no FMA contraction, IEEE div/sqrt, glibc libm, libstdc++ <random>.
 # The reference's own CMake build is not run (it needs Qt6 and FetchContent).
 set -euo pipefail
-REF="${MCSKIN_REFERENCE_DIR:-/root/reference}"
 HERE="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
 OUT="$HERE/_ref"
-if [ ! -d "$REF/src" ]; then
-    echo "build_ref.sh: $REF/src not found (expected off the build container); keeping any prebuilt $OUT" >&2
-    exit 0
+if [ -n "${MCSKIN_REFERENCE_DIR:-}" ]; then
+    REF="$MCSKIN_REFERENCE_DIR"
+    if [ ! -d "$REF/src" ]; then
+        echo "build_ref.sh: MCSKIN_REFERENCE_DIR=$REF is not a checkout of the reference (no src/)" >&2
+        exit 1
+    fi
+else
+    # default: a checkout named `reference` beside this repository; absent or unreadable means not present
+    REF="$HERE/../../reference"
+    if [ ! -d "$REF/src" ] || [ ! -r "$REF/src" ]; then
+        echo "build_ref.sh: no checkout of the reference at $REF (set MCSKIN_REFERENCE_DIR); keeping any prebuilt $OUT" >&2
+        exit 0
+    fi
 fi
 mkdir -p "$OUT/obj"
 CXX="${CXX:-g++}"

@@ -3,8 +3,9 @@
 * `Oracle`    : oracle/libmcskin_oracle.so, the plain-C restatement (mcskin_oracle.c).
                 Built on demand with gcc (present on the GPU box too).
 * `Reference` : oracle/_ref/libmcskin_ref.so, the UNMODIFIED reference core behind
-                ref_shim.cpp.  Built by oracle/build_ref.sh where /root/reference
-                exists; on the GPU box only the prebuilt .so is used.  None when absent.
+                ref_shim.cpp.  Built by oracle/build_ref.sh from a checkout of the
+                reference (not part of this repository): the one MCSKIN_REFERENCE_DIR
+                names, else `reference` beside this repository.  None when absent.
 
 Both expose the same operations on the flat PODs of include/mcskin_cuda.h.
 """
@@ -25,6 +26,8 @@ from minecraftskin_raytracer_b200.scene import FlatScene, pose_array
 HERE = Path(__file__).resolve().parent
 ORACLE_SO = HERE / "libmcskin_oracle.so"
 REF_SO = HERE / "_ref" / "libmcskin_ref.so"
+# where the reference is looked for when MCSKIN_REFERENCE_DIR is not set: a checkout named `reference` beside this repository
+DEFAULT_REFERENCE_DIR = HERE.parent.parent / "reference"
 
 COUNTER_FIELDS = [
     "n_intersect_scene", "n_primary_rays", "n_retests", "n_shadow_rays", "n_ao_rays", "n_reflect_rays",
@@ -71,11 +74,26 @@ def build_oracle(force: bool = False) -> Path:
     return ORACLE_SO
 
 
+def reference_dir() -> Path | None:
+    """The checkout of the reference to build the checker from: MCSKIN_REFERENCE_DIR when set (an error when it names
+    no checkout), else DEFAULT_REFERENCE_DIR when it holds one, else None."""
+    env = os.environ.get("MCSKIN_REFERENCE_DIR")
+    if env:
+        if not (Path(env) / "src").is_dir():
+            raise RuntimeError(f"MCSKIN_REFERENCE_DIR={env} is not a checkout of the reference (no src/)")
+        return Path(env)
+    try:
+        return DEFAULT_REFERENCE_DIR if (DEFAULT_REFERENCE_DIR / "src").is_dir() else None
+    except OSError:  # e.g. a parent directory this user may not enter: not present
+        return None
+
+
 def build_reference() -> Path | None:
-    """Compiles oracle/_ref when the reference tree is present; returns the .so path or None."""
-    ref_root = Path(os.environ.get("MCSKIN_REFERENCE_DIR", "/root/reference"))
-    if (ref_root / "src").is_dir():
-        subprocess.run(["bash", str(HERE / "build_ref.sh")], check=True, capture_output=True)
+    """Compiles oracle/_ref when a checkout of the reference is found (reference_dir); returns the .so path or None."""
+    ref = reference_dir()
+    if ref is not None:
+        subprocess.run(["bash", str(HERE / "build_ref.sh")], check=True, capture_output=True,
+                       env={**os.environ, "MCSKIN_REFERENCE_DIR": str(ref)})
     return REF_SO if REF_SO.exists() else None
 
 

@@ -1,13 +1,14 @@
 """Generates tests/golden/reference_vectors.npz from the UNMODIFIED reference
-(oracle/_ref/libmcskin_ref.so, built from /root/reference by oracle/build_ref.sh).
+(oracle/_ref/libmcskin_ref.so, built by oracle/build_ref.sh from the checkout that
+MCSKIN_REFERENCE_DIR names, else `reference` beside this repository).
 
 The reference ships no golden images (SURVEY.md §4), so these vectors are outputs of the
-reference itself run in the build container: small full-scene renders (float RGBA + the
-intersectScene call count), pixel-centre triangle ids, single-ray intersections, Blinn-Phong
-values, traced colours, soft-shadow / AO factors and the libstdc++ RNG streams behind them.
-They travel with the repo; /root/reference does not.
+reference itself: small full-scene renders (float RGBA + the intersectScene call count),
+pixel-centre triangle ids, single-ray intersections, Blinn-Phong values, traced colours,
+soft-shadow / AO factors and the libstdc++ RNG streams behind them.  They are committed
+so that the tests need no copy of the reference.
 
-    python tests/golden/make_golden.py
+    [MCSKIN_REFERENCE_DIR=<reference checkout>] python tests/golden/make_golden.py
 """
 import sys
 from pathlib import Path
@@ -37,7 +38,7 @@ def main():
     build_reference()
     ref = Reference.load()
     if ref is None:
-        raise SystemExit("oracle/_ref/libmcskin_ref.so is missing and /root/reference is not available")
+        raise SystemExit("oracle/_ref/libmcskin_ref.so is missing and no checkout of the reference was found (set MCSKIN_REFERENCE_DIR)")
     out = {}
     for name, seed, kind, pose, over in GOLDEN_RENDERS:
         atlas = synth_skin(seed, kind)

@@ -1,6 +1,6 @@
 """The reference's own hot-path unit tests, re-expressed once and run against every
 implementation of the path: the CPU oracle, the unmodified reference (oracle/_ref) and
-the CUDA library.  Each case cites the gtest it restates (/root/reference/tests/...).
+the CUDA library.  Each case cites the gtest it restates (the reference's tests/...).
 
 A backend offers: intersect(scene, rays, box=-1), shade(scene, cfg, hits, view_dirs, sf),
 in_shadow(scene, p, n, l), trace(scene, cfg, rays, depth, use_config),

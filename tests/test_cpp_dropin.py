@@ -1,8 +1,7 @@
 """The C++ drop-in layer (TileRenderer / RayTracer / intersect* over the C ABI):
-compiles against the re-authored headers and — when /root/reference is present — against the
-reference's own headers (CPU); on the GPU box the reference's TileRenderer tests, re-expressed
-in tests/cpp/dropin_test.cpp, run through it and its frame is compared with the oracle."""
-import os
+compiles against the re-authored headers and — when a checkout of the reference is found
+(oracle.harness.reference_dir) — against the reference's own headers (CPU); on a GPU the reference's TileRenderer tests,
+re-expressed in tests/cpp/dropin_test.cpp, run through it and its frame is compared with the oracle."""
 import subprocess
 from pathlib import Path
 
@@ -37,10 +36,11 @@ def test_dropin_layer_compiles_against_own_headers(mclib, tmp_path):
 
 
 def test_dropin_layer_compiles_against_reference_headers():
-    ref_src = Path(os.environ.get("MCSKIN_REFERENCE_DIR", "/root/reference")) / "src"
-    if not ref_src.is_dir():
-        pytest.skip("reference tree not present")
-    _compile([CORE / "tile_renderer.cpp", CORE / "raytracer_api.cpp"], None, [ROOT / "include", ref_src], link=False)
+    from oracle.harness import reference_dir
+    ref = reference_dir()
+    if ref is None:
+        pytest.skip("no checkout of the reference (MCSKIN_REFERENCE_DIR, or `reference` beside this repository)")
+    _compile([CORE / "tile_renderer.cpp", CORE / "raytracer_api.cpp"], None, [ROOT / "include", ref / "src"], link=False)
 
 
 @pytest.mark.gpu

@@ -10,8 +10,9 @@ import pytest
 
 from minecraftskin_raytracer_b200 import _abi
 from minecraftskin_raytracer_b200.scene import BUILTIN_POSE_ORDER, BUILTIN_POSES, FlatScene, pose_array, synth_skin
-from tests.golden_data import golden_scene, vectors
+from tests.golden_data import golden_scene, pins, vectors
 from tests.golden.make_golden import GOLDEN_RENDERS
+from tests.golden.make_oracle_pins import SCENE_SKINS, overlay_atlas, scene_digest
 from tests.scenes import make_config
 
 ROOT = Path(__file__).resolve().parent.parent
@@ -66,6 +67,21 @@ def test_skin_scene_builder_equals_live_reference(mclib, reference):
     poses = reference.builtin_poses()
     for i, name in enumerate(BUILTIN_POSE_ORDER):          # src/scene/pose.h:25-92
         assert np.array_equal(poses[i], pose_array(name)), name
+
+
+@pytest.mark.parametrize("seed,kind,pose", [(s, k, p) for s, k in SCENE_SKINS for p in [None] + BUILTIN_POSE_ORDER],
+                         ids=[f"{s}-{k}-{p}" for s, k in SCENE_SKINS for p in [None] + BUILTIN_POSE_ORDER])
+def test_skin_scene_builder_equals_pins(mclib, seed, kind, pose):
+    """The scenes of test_skin_scene_builder_equals_live_reference without the reference: equal to the digests in
+    tests/golden/oracle_pins.json (the builder's output, not the reference's)."""
+    assert scene_digest(mclib.build_skin_scene(synth_skin(seed, kind), pose)) == pins()["scenes"][f"{seed}/{kind}/{pose}"]
+
+
+def test_skin_scene_builder_drops_transparent_overlay(mclib):
+    """A fully transparent outer layer is dropped (mesh_builder.cpp:176-186); legacy skins keep 7 boxes."""
+    scene = mclib.build_skin_scene(overlay_atlas())
+    assert len(scene.boxes) == 11 and scene_digest(scene) == pins()["scenes"]["overlay_dropped"]
+    assert len(mclib.build_skin_scene(synth_skin(2, "legacy")).boxes) == 7
 
 
 def test_skin_layout_equals_the_scene_builder(mclib):

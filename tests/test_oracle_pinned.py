@@ -1,7 +1,7 @@
 """Pins the CPU oracle (oracle/mcskin_oracle.c) to the reference:
   * against committed outputs of the UNMODIFIED reference (tests/golden/reference_vectors.npz) —
-    always, including on the GPU box where /root/reference does not exist;
-  * against the unmodified reference itself (oracle/_ref) when it was built.
+    always, with no copy of the reference at hand;
+  * against the unmodified reference itself (oracle/_ref) when it was built (oracle.harness.reference_dir).
 Everything is required to match bit for bit: both are CPU code using the same glibc/libstdc++
 arithmetic, so any difference is a restatement error.
 """
@@ -9,7 +9,8 @@ import numpy as np
 import pytest
 
 from minecraftskin_raytracer_b200 import _abi
-from tests.golden_data import golden_render_cases, golden_scene, ray_scene, vectors
+from tests.golden.make_oracle_pins import digest, single_ray_inputs
+from tests.golden_data import golden_render_cases, golden_scene, pins, ray_scene, vectors
 from tests.scenes import RENDER_CASES, make_config, random_rays, synth_skin
 
 
@@ -88,6 +89,29 @@ def test_oracle_equals_live_reference_single_rays(oracle, reference):
     cfg = make_config(max_bounces=4, ao_enabled=1)
     assert np.array_equal(_bits(reference.trace(scene, cfg, rays[:800])), _bits(oracle.trace(scene, cfg, rays[:800])))
     assert reference.mt19937(77, 500)[0].tolist() == oracle.mt19937(77, 500)[0].tolist()
+
+
+@pytest.mark.parametrize("case", RENDER_CASES, ids=[c[0] for c in RENDER_CASES])
+def test_oracle_renders_equal_pins(oracle, mclib, case):
+    """The inputs of test_oracle_equals_live_reference without the reference: frame, intersectScene count and hit ids
+    equal the digests in tests/golden/oracle_pins.json (the oracle's outputs, not the reference's)."""
+    name, seed, kind, pose, over = case
+    want = pins()["renders"][name]
+    scene = mclib.build_skin_scene(synth_skin(seed, kind), pose)
+    cfg = make_config(**over)
+    img, cnt = oracle.render(scene, cfg, counters=True)
+    assert digest(img) == want["image"]
+    assert cnt["n_intersect_scene"] == want["calls"]
+    assert digest(oracle.aov(scene, cfg)) == want["tri_id"]
+
+
+def test_oracle_single_rays_equal_pins(oracle, mclib):
+    """The inputs of test_oracle_equals_live_reference_single_rays (4 bounces, AO on) without the reference."""
+    want = pins()["rays"]
+    scene, rays, cfg = single_ray_inputs(mclib.build_skin_scene)
+    assert digest(oracle.intersect(scene, rays)) == want["hits"]
+    assert digest(oracle.trace(scene, cfg, rays[:800])) == want["trace"]
+    assert digest(oracle.mt19937(77, 500)[0]) == want["mt19937_77"]
 
 
 def test_render_tile_equals_render(oracle, mclib):
