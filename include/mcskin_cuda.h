@@ -167,6 +167,27 @@ int32_t mcskin_cuda_render(const McScene* scene, const McConfig* cfg, int32_t de
                            float* out_rgba_f32, uint8_t* out_rgba_u8,
                            McProgressFn progress, void* user, McRenderStats* stats);
 
+/* Per-pixel planes rendered in the same pass as the colour ("AOVs"), each width*height values indexed like the colour
+ * image of the same call; any member may be NULL.  For pixel (px, py) with samples s = 0..spp-1 in the renderer's sample
+ * order, let h_s be the closest hit of sample s's camera ray exactly as the colour pass builds it (jitter, thin lens,
+ * either rng_mode; the query whose miss gives the sample the gradient, tile_renderer.cpp:111), and n the number of
+ * samples that hit.  Independent of max_bounces, shading, shadows and AO:
+ *   coverage : (float)n * (1.0f / (float)spp)
+ *   depth    : the hit distances h_s.t of the hitting samples summed left to right from 0.0f, divided by (float)n;
+ *              0.0f when n == 0
+ *   tri_id   : box*12 + face*2 of the first hitting sample (the McHit / mcskin_cuda_aov convention); -1 when n == 0 */
+typedef struct McAovTargets {
+    float* coverage;
+    float* depth;
+    int32_t* tri_id;
+} McAovTargets;
+
+/* mcskin_cuda_render with AOV planes: the same colour bytes, and the planes `aov` asks for (host memory, width*height
+ * values each; aov may be NULL).  A frame with no tiles leaves the defaults (0, 0, -1) in every requested plane. */
+int32_t mcskin_cuda_render_aovs(const McScene* scene, const McConfig* cfg, int32_t device,
+                                float* out_rgba_f32, uint8_t* out_rgba_u8, const McAovTargets* aov,
+                                McRenderStats* stats);
+
 /* TileRenderer::renderTile (tile_renderer.cpp:71-127): renders one tile into the
  * caller's full-size image buffers (only the tile's pixels are written). */
 int32_t mcskin_cuda_render_tile(const McScene* scene, const McConfig* cfg, int32_t device,
@@ -258,6 +279,12 @@ int32_t mcskin_cuda_peer_wait(int32_t device, const void* d_flags, int32_t n, ui
  * kernels record when they ran: 4 words per block (entry ns, exit ns, frame tile, part | parts << 16; zeros for
  * blocks that had nothing to do).  Returns the number of records of the last launch. */
 int32_t mcskin_cuda_context_debug_block_times(McContext* ctx, uint64_t* out, int32_t capacity);
+/* AOV planes for the context's later render calls: d_targets holds DEVICE-addressable pointers (copied; NULL, or all
+ * members NULL, switches the planes off).  render_bands, render_rows_into_frame, render_tiles_into_frame, render_batch and
+ * render_skin_batch then write every plane that is set for every pixel they render, at the colour image's index (image i
+ * of a batch at offset i*width*height); frame lanes inherit the targets.  render_scene_tiles fails with MC_ERR_INVALID
+ * while targets are set. */
+int32_t mcskin_cuda_context_set_aov_targets(McContext* ctx, const McAovTargets* d_targets);
 /* Blocks until the context's work is done, fills stats of the last render. */
 int32_t mcskin_cuda_context_sync(McContext* ctx, McRenderStats* stats);
 /* Tuning / test knobs (every combination renders the same bits; INTEGRATION.md §6 has the table):

@@ -98,6 +98,11 @@ class McRenderStats(C.Structure):
     ]
 
 
+class McAovTargets(C.Structure):
+    """Per-pixel planes rendered next to the colour (include/mcskin_cuda.h); null members are not written."""
+    _fields_ = [("coverage", C.c_void_p), ("depth", C.c_void_p), ("tri_id", C.c_void_p)]
+
+
 class McRay(C.Structure):
     _fields_ = [("origin", C.c_float * 3), ("dir", C.c_float * 3)]
 

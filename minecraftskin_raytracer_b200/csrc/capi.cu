@@ -161,6 +161,7 @@ struct McContext {
         unsigned long long mapVersion;
         int nTiles, nHeavy;
         const void *hotF32, *hotU8;
+        const void *aovCoverage, *aovDepth, *aovTriId;  // a graph with AOV stores is never replayed without them, or vice versa
         long long optionBits[12];
         unsigned long long allocEpoch;
         bool operator==(const GraphKey& o) const { return std::memcmp(this, &o, sizeof(GraphKey)) == 0; }
@@ -202,9 +203,23 @@ struct McContext {
     cudaEvent_t evStage[2] = {nullptr, nullptr};
     std::vector<PreparedFrame> batchPreps;
     std::vector<McContext*> lanes;
+    // AOV planes the render calls write next to the colour (mcskin_cuda_context_set_aov_targets; device-addressable
+    // pointers, all null: none).  Child lanes get their parent's (inherit_options).
+    McAovTargets aov{};
+    DevBuf aovPlanes;                        // mcskin_cuda_render_aovs: the planes on the device before they go to the host
 };
 
 namespace {
+
+bool aov_on(const McContext* ctx) { return ctx->aov.coverage || ctx->aov.depth || ctx->aov.tri_id; }
+// the planes of the image that starts `pixels` pixels into the targets (image i of a batch)
+McAovTargets aov_at(const McAovTargets& a, size_t pixels) {
+    McAovTargets r{};
+    r.coverage = a.coverage ? a.coverage + pixels : nullptr;
+    r.depth = a.depth ? a.depth + pixels : nullptr;
+    r.tri_id = a.tri_id ? a.tri_id + pixels : nullptr;
+    return r;
+}
 
 int upload_scene(McContext* ctx) {
     const PreparedFrame& pf = ctx->prep;
@@ -378,8 +393,11 @@ int render_bands_lane(McContext* ctx, const McContext* scn, const BandSpec& spec
     // less than 1.25 entries per path; paths whose hits do not fit are redone in-thread), then the number of
     // paths does (pixels beyond them are shaded by the megakernel).
     WaveView wave{};
+    const bool aov = aov_on(ctx);
+    AovView aovView{};
+    aovView.planes = ctx->aov;
     if (ctx->shadeMode == 0) {
-        const size_t perPath = wavefront_bytes_per_path(f), perEntry = wavefront_bytes_per_entry();
+        const size_t perPath = wavefront_bytes_per_path(f, aov), perEntry = wavefront_bytes_per_entry();
         const size_t hitsMax = static_cast<size_t>(wavefront_max_hits_per_path(f));
         const size_t budget = static_cast<size_t>(ctx->waveBudgetBytes);
         const size_t worstPaths = slotCap * static_cast<size_t>(f.spp);
@@ -394,7 +412,7 @@ int render_bands_lane(McContext* ctx, const McContext* scn, const BandSpec& spec
         const size_t bytes = paths * perPath + entries * perEntry + wavefront_fixed_bytes(f) + 16 * 256;
         CU_TRY(ctx->wave.reserve(bytes));
         if (!wavefront_carve(f, ctx->wave.p, ctx->wave.cap, static_cast<unsigned int>(paths), static_cast<unsigned int>(entries),
-                             ctx->smCount * ctx->shadeBlocksPerSm, &wave))
+                             ctx->smCount * ctx->shadeBlocksPerSm, &wave, aov ? &aovView : nullptr))
             return fail(MC_ERR_CUDA, "wavefront buffer carve failed");
         wave.softGrid = ctx->smCount * ctx->softBlocksPerSm;
         wave.seedMemo = static_cast<uint2*>(scn->seedMemo.p);  // (render_bands has seen to it; the lanes of a frame share it)
@@ -458,6 +476,10 @@ int render_bands_lane(McContext* ctx, const McContext* scn, const BandSpec& spec
             CU_TRY(cudaMemcpyAsync(list.count, &list.capacity, sizeof(unsigned int), cudaMemcpyHostToDevice, stream));
         }
         if (!ctx->capturing) CU_TRY(cudaEventRecord(ctx->passEvents[3 * c], stream));
+        if (aov) {  // every pixel of the chunk gets the defaults; the shading pass overwrites the ones it resolves
+            launch_aov_defaults(f, band, ctx->aov, nullptr, 1, stream);
+            ++launches;
+        }
         // (three builds of the kernels — dev_types.cuh: counter-based random streams; no pose code, for scenes in which
         // no box is posed; the general form)
         const int build = f.rng_mode ? 2 : (f.any_rotated ? 0 : 1);
@@ -476,14 +498,13 @@ int render_bands_lane(McContext* ctx, const McContext* scn, const BandSpec& spec
         unsigned int* groupCounter = static_cast<unsigned int*>(ctx->countLog.p) + nChunks + c;
         const int shadeGrid = ctx->smCount * ctx->shadeBlocksPerSm;
         if (ctx->shadeMode == 0) {
-            if (build == 2) counter::launch_wavefront(f, fp, band, list, wave, groupCounter, stream, &launches);
-            else if (build == 1) plain::launch_wavefront(f, fp, band, list, wave, groupCounter, stream, &launches);
-            else launch_wavefront(f, fp, band, list, wave, groupCounter, stream, &launches);
+            if (build == 2) counter::launch_wavefront(f, fp, band, list, wave, groupCounter, stream, &launches, nullptr, 1, aov ? &aovView : nullptr);
+            else if (build == 1) plain::launch_wavefront(f, fp, band, list, wave, groupCounter, stream, &launches, nullptr, 1, aov ? &aovView : nullptr);
+            else launch_wavefront(f, fp, band, list, wave, groupCounter, stream, &launches, nullptr, 1, aov ? &aovView : nullptr);
         } else {
-            if (build == 2) counter::launch_shade(f, fp, band, list, shadeGrid, groupCounter, 0u, stream, ctx->shadeMode);
-            else if (build == 1) plain::launch_shade(f, fp, band, list, shadeGrid, groupCounter, 0u, stream, ctx->shadeMode);
-            else launch_shade(f, fp, band, list, shadeGrid, groupCounter, 0u, stream, ctx->shadeMode);
-            ++launches;
+            if (build == 2) launches += counter::launch_shade(f, fp, band, list, shadeGrid, groupCounter, 0u, stream, ctx->shadeMode, &ctx->aov);
+            else if (build == 1) launches += plain::launch_shade(f, fp, band, list, shadeGrid, groupCounter, 0u, stream, ctx->shadeMode, &ctx->aov);
+            else launches += launch_shade(f, fp, band, list, shadeGrid, groupCounter, 0u, stream, ctx->shadeMode, &ctx->aov);
         }
         if (!ctx->capturing) CU_TRY(cudaEventRecord(ctx->passEvents[3 * c + 2], stream));
         ++launches;
@@ -520,6 +541,7 @@ void inherit_options(McContext* lane, const McContext* ctx) {
     lane->primaryBlocksPerSm = ctx->primaryBlocksPerSm;
     lane->heavyTilesPerSm = ctx->heavyTilesPerSm;
     lane->cacheTileSeeds = ctx->cacheTileSeeds;
+    lane->aov = ctx->aov;
     lane->useGraphs = 0;
 }
 
@@ -604,6 +626,7 @@ int render_bands(McContext* ctx, int first, int stride, float4* outF32, uchar4* 
         key.blobBytes = static_cast<unsigned int>(ctx->prep.blob.size());
         key.first = first; key.stride = stride; key.lanes = L * 2 + (frameLayout ? 1 : 0);
         key.hotF32 = hotF32; key.hotU8 = hotU8;
+        key.aovCoverage = ctx->aov.coverage; key.aovDepth = ctx->aov.depth; key.aovTriId = ctx->aov.tri_id;
         if (tiles) {
             key.tileMap = tiles->map; key.mapVersion = tiles->mapVersion; key.nTiles = tiles->nTiles; key.nHeavy = tiles->nHeavy;
         }
@@ -956,7 +979,8 @@ int render_batch_grouped(McContext* ctx, const McScene* scenes, const SkinBatchS
     const size_t recordBytes = std::max<size_t>(16, slotCap * f0.spp * f0.draws_per_sample * sizeof(float));
     const size_t entries = paths * static_cast<size_t>(wavefront_max_hits_per_path(f0));  // cannot overflow
     if (entries > 0xffffff00u) return MC_OK;
-    const size_t waveBytes = (paths * wavefront_bytes_per_path(f0) + entries * wavefront_bytes_per_entry() +
+    const bool aov = aov_on(ctx);
+    const size_t waveBytes = (paths * wavefront_bytes_per_path(f0, aov) + entries * wavefront_bytes_per_entry() +
                               wavefront_fixed_bytes(f0) + 16 * 256 + 255) & ~size_t(255);
     const size_t perScene = waveBytes + recordBytes + slotCap * sizeof(uint2);
     int G = std::min<int>(ctx->batchGroup, nScenes);
@@ -981,7 +1005,9 @@ int render_batch_grouped(McContext* ctx, const McScene* scenes, const SkinBatchS
         sceneStride = std::max(sceneStride, blob + tex);
     }
     if (sceneStride > (8u << 20)) return MC_OK;
-    CU_TRY(ctx->batchScenes.reserve(static_cast<size_t>(G) * (sceneStride + sizeof(BatchSlice))));
+    // per scene: its data, its slice, its AOV view
+    const size_t perSceneStage = sceneStride + sizeof(BatchSlice) + sizeof(AovView);
+    CU_TRY(ctx->batchScenes.reserve(static_cast<size_t>(G) * perSceneStage));
     CU_TRY(ctx->batchSlots.reserve(static_cast<size_t>(G) * slotCap * sizeof(uint2)));
     CU_TRY(ctx->batchRecords.reserve(static_cast<size_t>(G) * recordBytes));
     CU_TRY(ctx->batchWave.reserve(static_cast<size_t>(G) * waveBytes));
@@ -989,7 +1015,7 @@ int render_batch_grouped(McContext* ctx, const McScene* scenes, const SkinBatchS
     CU_TRY(ctx->batchCounts.reserve(static_cast<size_t>(G) * sizeof(unsigned int)));
     CU_TRY(ctx->tileStates.reserve(std::max<size_t>(16, static_cast<size_t>(f0.tiles_x) * f0.tiles_y * 624 * sizeof(uint32_t) *
                                                             static_cast<size_t>(primary_states_per_tile(f0, f0.tiles_x * f0.tiles_y, 1, ctx->smCount * ctx->primaryBlocksPerSm, 0)))));
-    for (int i = 0; i < 2; ++i) CU_TRY(ctx->batchStage[i].reserve(static_cast<size_t>(G) * (sceneStride + sizeof(BatchSlice))));
+    for (int i = 0; i < 2; ++i) CU_TRY(ctx->batchStage[i].reserve(static_cast<size_t>(G) * perSceneStage));
     if (skins) {
         CU_TRY(ctx->batchSkinSrc.reserve(static_cast<size_t>(G) * skinRecord));
         for (int i = 0; i < 2; ++i) CU_TRY(ctx->batchSkinStage[i].reserve(static_cast<size_t>(G) * skinRecord));
@@ -1000,7 +1026,8 @@ int render_batch_grouped(McContext* ctx, const McScene* scenes, const SkinBatchS
     ++ctx->seedGen;
 
     unsigned char* devScenes = static_cast<unsigned char*>(ctx->batchScenes.p);
-    const size_t sliceOffset = static_cast<size_t>(G) * sceneStride;  // slices follow the scene data
+    const size_t sliceOffset = static_cast<size_t>(G) * sceneStride;  // slices follow the scene data, AOV views the slices
+    const size_t aovOffset = sliceOffset + static_cast<size_t>(G) * sizeof(BatchSlice);
     int stageSlot = 0;
     bool seeded = false;
     int seededStatesPerTile = 0;
@@ -1063,6 +1090,7 @@ int render_batch_grouped(McContext* ctx, const McScene* scenes, const SkinBatchS
         // stage: scene data at slot i (chunk-local index), slices ordered group by group
         unsigned char* stage = static_cast<unsigned char*>(ctx->batchStage[stageSlot].p);
         BatchSlice* stageSlices = reinterpret_cast<BatchSlice*>(stage + sliceOffset);
+        AovView* stageAovs = reinterpret_cast<AovView*>(stage + aovOffset);
         int sliceAt = 0;
         std::vector<int> groupFirstSlice(groups.size(), 0);
         for (size_t g = 0; g < groups.size(); ++g) {
@@ -1084,6 +1112,8 @@ int render_batch_grouped(McContext* ctx, const McScene* scenes, const SkinBatchS
                 sl.band.out_row_stride = 1;
                 sl.band.out_f32 = outF32 ? outF32 + static_cast<size_t>(c0 + i) * pixels : nullptr;
                 sl.band.out_u8 = outU8 ? outU8 + static_cast<size_t>(c0 + i) * pixels : nullptr;
+                AovView av{};
+                av.planes = aov_at(ctx->aov, static_cast<size_t>(c0 + i) * pixels);
                 sl.list.count = static_cast<unsigned int*>(ctx->batchCounts.p) + i;
                 sl.list.slot_pixel = static_cast<uint2*>(ctx->batchSlots.p) + static_cast<size_t>(i) * slotCap;
                 sl.list.records = reinterpret_cast<float*>(static_cast<unsigned char*>(ctx->batchRecords.p) + static_cast<size_t>(i) * recordBytes);
@@ -1092,9 +1122,10 @@ int render_batch_grouped(McContext* ctx, const McScene* scenes, const SkinBatchS
                 // few blocks per scene: a launch has gridDim.y scenes to fill the machine with
                 const int gridX = std::max(2, (ctx->smCount * ctx->shadeBlocksPerSm + nC - 1) / nC);
                 if (!wavefront_carve(pf.frame, static_cast<unsigned char*>(ctx->batchWave.p) + static_cast<size_t>(i) * waveBytes,
-                                     waveBytes, static_cast<unsigned int>(paths), static_cast<unsigned int>(entries), gridX, &sl.wave))
+                                     waveBytes, static_cast<unsigned int>(paths), static_cast<unsigned int>(entries), gridX, &sl.wave, aov ? &av : nullptr))
                     return MC_OK;  // (cannot happen: the sizes depend on the config only) frame-by-frame path instead
                 sl.wave.seedMemo = batchSeedMemo;
+                stageAovs[sliceAt] = av;
                 stageSlices[sliceAt++] = sl;
             }
         }
@@ -1110,15 +1141,21 @@ int render_batch_grouped(McContext* ctx, const McScene* scenes, const SkinBatchS
         }
         CU_TRY(cudaMemcpyAsync(devScenes + sliceOffset, stage + sliceOffset, static_cast<size_t>(nC) * sizeof(BatchSlice),
                                cudaMemcpyHostToDevice, stream));
+        if (aov)
+            CU_TRY(cudaMemcpyAsync(devScenes + aovOffset, stage + aovOffset, static_cast<size_t>(nC) * sizeof(AovView),
+                                   cudaMemcpyHostToDevice, stream));
         CU_TRY(cudaEventRecord(ctx->evStage[stageSlot], stream));
         stageSlot ^= 1;
         const BatchSlice* devSlices = reinterpret_cast<const BatchSlice*>(devScenes + sliceOffset);
+        const AovView* devAovs = aov ? reinterpret_cast<const AovView*>(devScenes + aovOffset) : nullptr;
         for (size_t g = 0; g < groups.size(); ++g) {
             const int nS = static_cast<int>(groups[g].size());
             const BatchSlice* gs = devSlices + groupFirstSlice[g];
+            const AovView* gAov = devAovs ? devAovs + groupFirstSlice[g] : nullptr;
             const BatchSlice& first = stageSlices[groupFirstSlice[g]];
             const DevFrame& f = ctx->batchPreps[groups[g][0]].frame;
             launch_batch_reset(gs, nS, stream);
+            if (gAov) launch_aov_defaults(f, first.band, McAovTargets{}, gAov, nS, stream);
             const int build = f.rng_mode ? 2 : (f.any_rotated ? 0 : 1);  // (equal frame descriptions: equal for the whole group)
             // the engines are seeded once per batch — same image geometry for every scene — unless a group is small enough
             // for its tiles to be split over blocks, which changes what is kept per tile
@@ -1134,9 +1171,9 @@ int render_batch_grouped(McContext* ctx, const McScene* scenes, const SkinBatchS
             seeded = true;
             seededStatesPerTile = statesPerTile;
             int launches = 0;
-            if (build == 2) counter::launch_wavefront(f, first.fp, first.band, first.list, first.wave, nullptr, stream, &launches, gs, nS);
-            else if (build == 1) plain::launch_wavefront(f, first.fp, first.band, first.list, first.wave, nullptr, stream, &launches, gs, nS);
-            else launch_wavefront(f, first.fp, first.band, first.list, first.wave, nullptr, stream, &launches, gs, nS);
+            if (build == 2) counter::launch_wavefront(f, first.fp, first.band, first.list, first.wave, nullptr, stream, &launches, gs, nS, nullptr, gAov);
+            else if (build == 1) plain::launch_wavefront(f, first.fp, first.band, first.list, first.wave, nullptr, stream, &launches, gs, nS, nullptr, gAov);
+            else launch_wavefront(f, first.fp, first.band, first.list, first.wave, nullptr, stream, &launches, gs, nS, nullptr, gAov);
         }
         CU_TRY(cudaGetLastError());
     }
@@ -1227,7 +1264,8 @@ void mcskin_cuda_context_destroy(McContext* ctx) {
         if (ctx->evStage[i]) cudaEventDestroy(ctx->evStage[i]);
         ctx->batchStage[i].release();
     }
-    for (DevBuf* b : {&ctx->batchScenes, &ctx->batchSlots, &ctx->batchRecords, &ctx->batchWave, &ctx->batchCounts, &ctx->batchSkinSrc}) b->release();
+    for (DevBuf* b : {&ctx->batchScenes, &ctx->batchSlots, &ctx->batchRecords, &ctx->batchWave, &ctx->batchCounts, &ctx->batchSkinSrc,
+                      &ctx->aovPlanes}) b->release();
     for (int i = 0; i < 2; ++i) ctx->batchSkinStage[i].release();
     if (ctx->copyStream) cudaStreamDestroy(ctx->copyStream);
     if (ctx->evUpload) cudaEventDestroy(ctx->evUpload);
@@ -1428,6 +1466,7 @@ static int finish_tiles_to_host(McContext* ctx) {
 int32_t mcskin_cuda_context_render_scene_tiles(McContext* ctx, const McScene* scene, const McConfig* cfg, const int32_t* tiles,
                                                 int32_t nTiles, float* hostF32, uint8_t* hostU8, float* msDevice) {
     if (!ctx) return fail(MC_ERR_INVALID, "render_scene_tiles: null context");
+    if (aov_on(ctx)) return fail(MC_ERR_INVALID, "render_scene_tiles: writes no AOV planes; switch the context's AOV targets off first");
     if (nTiles < 0 || (nTiles > 0 && !tiles)) return fail(MC_ERR_INVALID, "render_scene_tiles: bad tile list");
     int rc = mcskin_cuda_context_set_scene(ctx, scene, cfg);
     if (rc != MC_OK) return rc;
@@ -1753,6 +1792,48 @@ int32_t mcskin_cuda_render(const McScene* scene, const McConfig* cfg, int32_t de
     return MC_OK;
 }
 
+int32_t mcskin_cuda_render_aovs(const McScene* scene, const McConfig* cfg, int32_t device, float* outF32, uint8_t* outU8,
+                                const McAovTargets* aov, McRenderStats* stats) {
+    if (!scene || !cfg) return fail(MC_ERR_INVALID, "render_aovs: null scene or config");
+    const size_t pixels = cfg->width > 0 && cfg->height > 0 ? static_cast<size_t>(cfg->width) * cfg->height : 0;
+    const McAovTargets want = aov ? *aov : McAovTargets{};
+    const int32_t totalTiles = mcskin_generate_tiles(cfg->width, cfg->height, cfg->tile_size, nullptr, 0);
+    if (totalTiles == 0) {  // nothing is rendered: every plane keeps its defaults
+        if (want.coverage) std::fill(want.coverage, want.coverage + pixels, 0.0f);
+        if (want.depth) std::fill(want.depth, want.depth + pixels, 0.0f);
+        if (want.tri_id) std::fill(want.tri_id, want.tri_id + pixels, -1);
+        if (stats) *stats = McRenderStats{};
+        return MC_OK;
+    }
+    std::lock_guard<std::mutex> lock(g_ctxMutex);
+    McContext* ctx = nullptr;
+    int rc = shared_context(device, &ctx);
+    if (rc != MC_OK) return rc;
+    CU_TRY(cudaSetDevice(ctx->device));
+    CU_TRY(ctx->aovPlanes.reserve(std::max<size_t>(16, pixels * 3 * sizeof(float))));
+    float* const base = static_cast<float*>(ctx->aovPlanes.p);
+    McAovTargets dev{};
+    dev.coverage = want.coverage ? base : nullptr;
+    dev.depth = want.depth ? base + pixels : nullptr;
+    dev.tri_id = want.tri_id ? reinterpret_cast<int32_t*>(base + 2 * pixels) : nullptr;
+    ctx->aov = dev;
+    rc = render_host(ctx, scene, cfg, 0, 1, outF32, outU8, 0, stats);
+    ctx->aov = McAovTargets{};
+    if (rc != MC_OK) return rc;
+    // (render_host has synchronised with the frame)
+    if (want.coverage) CU_TRY(cudaMemcpyAsync(want.coverage, dev.coverage, pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    if (want.depth) CU_TRY(cudaMemcpyAsync(want.depth, dev.depth, pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    if (want.tri_id) CU_TRY(cudaMemcpyAsync(want.tri_id, dev.tri_id, pixels * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CU_TRY(cudaStreamSynchronize(ctx->stream));
+    return MC_OK;
+}
+
+int32_t mcskin_cuda_context_set_aov_targets(McContext* ctx, const McAovTargets* dTargets) {
+    if (!ctx) return fail(MC_ERR_INVALID, "set_aov_targets: null context");
+    ctx->aov = dTargets ? *dTargets : McAovTargets{};
+    return MC_OK;
+}
+
 int32_t mcskin_cuda_render_tile(const McScene* scene, const McConfig* cfg, int32_t device, const McTile* tile,
                                 float* imageF32, uint8_t* imageU8) {
     if (!scene || !cfg || !tile) return fail(MC_ERR_INVALID, "render_tile: null argument");
@@ -1881,6 +1962,7 @@ int32_t mcskin_cuda_context_render_batch(McContext* ctx, const McScene* scenes, 
         McContext* lane = ctx->lanes[i % nLanes];
         int rc = mcskin_cuda_context_set_scene(lane, &scenes[i], cfg);
         if (rc != MC_OK) return rc;
+        lane->aov = aov_at(ctx->aov, static_cast<size_t>(i) * pixels);
         rc = render_bands(lane, 0, 1, dOutF32 ? static_cast<float4*>(dOutF32) + i * pixels : nullptr,
                           dOutU8 ? static_cast<uchar4*>(dOutU8) + i * pixels : nullptr, lane->stream);
         if (rc != MC_OK) return rc;
@@ -1935,9 +2017,12 @@ int32_t mcskin_cuda_context_render_skin_batch(McContext* ctx, const uint8_t* atl
                                          texels.data() + static_cast<size_t>(i) * (kSkinMaxTexels + 16) * 4, &scenes[i]);
             if (rc != MC_OK) return rc;
         }
+        const McAovTargets planes = ctx->aov;  // (the chunk's images start c0 images in)
+        ctx->aov = aov_at(planes, static_cast<size_t>(c0) * pixels);
         rc = mcskin_cuda_context_render_batch(ctx, scenes.data(), n, cfg,
                                               dOutF32 ? static_cast<float4*>(dOutF32) + static_cast<size_t>(c0) * pixels : nullptr,
                                               dOutU8 ? static_cast<uchar4*>(dOutU8) + static_cast<size_t>(c0) * pixels : nullptr, caller);
+        ctx->aov = planes;
         if (rc != MC_OK) return rc;
         // the host arrays are reused by the next chunk: the uploads above are staged synchronously (pageable sources)
     }

@@ -65,6 +65,27 @@ __device__ __forceinline__ void store_pixel(const BandView& band, unsigned int i
     if (band.out_u8) band.out_u8[index] = quantize4(c);
 }
 
+// The AOV planes of a pixel (McAovTargets), folded over its samples' camera-ray hits (the query whose miss gives a
+// sample the gradient, tile_renderer.cpp:111) in sample order: hit count, left-to-right sum of the hit distances,
+// id of the first hit.  store_aov writes them at the index store_pixel uses; a fold without hits gives (0, 0, -1).
+struct AovFold {
+    int n = 0;
+    float tsum = 0.0f;
+    int id = -1;
+    __device__ __forceinline__ void add(float t, int hitId) {
+        if (hitId < 0) return;
+        if (n == 0) id = hitId;
+        ++n;
+        tsum += t;
+    }
+};
+__device__ __forceinline__ int aov_id(const Hit& h) { return h.box >= 0 ? h.box * 12 + h.face * 2 : -1; }  // McHit / k_aov
+__device__ __forceinline__ void store_aov(const DevFrame& fr, const McAovTargets& planes, unsigned int index, const AovFold& a) {
+    if (planes.coverage) planes.coverage[index] = static_cast<float>(a.n) * fr.inv_spp;
+    if (planes.depth) planes.depth[index] = a.n > 0 ? a.tsum / static_cast<float>(a.n) : 0.0f;
+    if (planes.tri_id) planes.tri_id[index] = a.id;
+}
+
 __device__ __forceinline__ float4 add4(float4 a, float4 b) {
     return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);
 }

@@ -1056,6 +1056,55 @@ k_shade_warp(const DevFrame fr, const FramePointers fp, const BandView band, con
     }
 }
 
+// ------------------------------------------------------------------ AOV planes
+// Every pixel of the band's tiles gets the defaults (launch_aov_defaults); blockIdx.x = tile, blockIdx.y = scene.
+template <bool BATCH>
+__global__ void __launch_bounds__(kBlockThreads)
+k_aov_defaults(const DevFrame fr, const BandView band, const McAovTargets planes_, const AovView* __restrict__ aovBatch) {
+    const McAovTargets& planes = BATCH ? aovBatch[blockIdx.y].planes : planes_;  // (every scene's band has the same tiles)
+    const TileGeom tg = tile_geom(fr, band, blockIdx.x);
+    const int nPix = tg.w * tg.h;
+    for (int q = threadIdx.x; q < nPix; q += kBlockThreads) {
+        const int ly = q / tg.w, lx = q - ly * tg.w;
+        store_aov(fr, planes, static_cast<unsigned int>(tg.bandRow0 + ly) * static_cast<unsigned int>(fr.width) + (tg.x + lx), AovFold{});
+    }
+}
+
+// The planes of the listed pixels from `firstSlot` on, for the megakernel forms of the shading pass (which stay as
+// they are: frames without AOV planes run exactly the same kernels): one thread per pixel builds every sample's camera
+// ray from the work record as k_shade_cta / k_shade_warp do and folds the closest hits in sample order.
+__global__ void __launch_bounds__(kBlockThreads)
+k_aov_listed(const DevFrame fr, const FramePointers fp, const ActiveList list, const unsigned int firstSlot,
+             const McAovTargets planes) {
+    unsigned int count = *list.count;
+    if (count > list.capacity) count = list.capacity;
+    const SceneView sc = scene_view(fp.blob, fp.texels, fr);
+    const int spp = fr.spp, dps = fr.draws_per_sample;
+    for (unsigned int slot = firstSlot + blockIdx.x * kBlockThreads + threadIdx.x; slot < count; slot += gridDim.x * kBlockThreads) {
+        const uint2 sp = list.slot_pixel[slot];
+        if (sp.x == kUnusedSlot) continue;
+        const int px = static_cast<int>(sp.y & 0xffffu), py = static_cast<int>(sp.y >> 16);
+        AovFold a;
+        for (int s = 0; s < spp; ++s) {
+            float d0 = 0.0f, d1 = 0.0f, d2 = 0.0f, d3 = 0.0f;
+            const float* rec = list.records + (static_cast<size_t>(slot) * spp + s) * dps;
+            if (dps == 2) {
+                const float2 r = *reinterpret_cast<const float2*>(rec);
+                d0 = r.x; d1 = r.y;
+            } else if (dps == 4) {
+                const float4 r = *reinterpret_cast<const float4*>(rec);
+                d0 = r.x; d1 = r.y; d2 = r.z; d3 = r.w;
+            }
+            const SampleDraws sd = assign_draws(fr, d0, d1, d2, d3);
+            float u, v;
+            sample_uv(fr, px, py, sd, &u, &v);
+            const Hit h = closest_hit(sc, primary_ray(fr, u, v, sd));
+            a.add(h.t, aov_id(h));
+        }
+        store_aov(fr, planes, sp.x, a);
+    }
+}
+
 // ------------------------------------------------------------------ single-query kernels
 __device__ __forceinline__ void write_hit(const SceneView& sc, const Hit& h, McHit* o) {
     McHit r;
@@ -1371,14 +1420,26 @@ bool launch_primary_batch(const DevFrame& fr, const BandView& band, uint32_t* ti
     return true;
 }
 
-void launch_shade(const DevFrame& fr, const FramePointers& fp, const BandView& band, const ActiveList& list,
-                  int gridBlocks, unsigned int* groupCounter, unsigned int firstSlot, cudaStream_t stream, int variant) {
-    if (gridBlocks <= 0) return;
+int launch_shade(const DevFrame& fr, const FramePointers& fp, const BandView& band, const ActiveList& list,
+                 int gridBlocks, unsigned int* groupCounter, unsigned int firstSlot, cudaStream_t stream, int variant,
+                 const McAovTargets* aov) {
+    if (gridBlocks <= 0) return 0;
     const int lg = log2_if_warp_spp(fr.spp);
     if (variant == 2 && lg >= 0)
         k_shade_warp<<<gridBlocks, kBlockThreads, fp.blob_bytes, stream>>>(fr, fp, band, list, lg, groupCounter, firstSlot);
     else
         k_shade_cta<<<gridBlocks, kBlockThreads, fp.blob_bytes, stream>>>(fr, fp, band, list, firstSlot);
+    if (!aov_any(aov)) return 1;
+    k_aov_listed<<<gridBlocks, kBlockThreads, 0, stream>>>(fr, fp, list, firstSlot, *aov);
+    return 2;
+}
+
+void launch_aov_defaults(const DevFrame& fr, const BandView& band, const McAovTargets& planes, const AovView* aovBatch, int nScenes,
+                         cudaStream_t stream) {
+    const int nTiles = band_tile_count(band, fr.tiles_x);
+    if (nTiles <= 0 || nScenes <= 0) return;
+    if (aovBatch) k_aov_defaults<true><<<dim3(nTiles, nScenes), kBlockThreads, 0, stream>>>(fr, band, planes, aovBatch);
+    else k_aov_defaults<false><<<nTiles, kBlockThreads, 0, stream>>>(fr, band, planes, aovBatch);
 }
 
 void launch_intersect(const DevFrame& fr, const FramePointers& fp, int box, const McRay* rays, int n, McHit* out,

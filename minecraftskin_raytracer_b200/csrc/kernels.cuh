@@ -88,6 +88,10 @@ struct BandView {
 __host__ __device__ inline int band_tile_count(const BandView& band, int tilesX) {
     return band.tile_map ? band.n_tiles : band.n_tile_rows * tilesX;
 }
+// AOV planes (McAovTargets, device pointers) travel next to a BandView, indexed like its out_f32: the launchers pick the
+// AOV instantiations of the shading kernels when any plane is set, and the kernels of frames without run as before.
+// (Not members of BandView: the batched primary kernels copy a scene's BandView, and a larger one costs them registers.)
+__host__ __device__ inline bool aov_any(const McAovTargets* a) { return a && (a->coverage || a->depth || a->tri_id); }
 
 // Work list produced by the primary pass for the shading pass.
 struct ActiveList {
@@ -110,9 +114,9 @@ struct FramePointers {
     bool launch_primary(const DevFrame& fr, const FramePointers& fp, const BandView& band, const ActiveList& list,      \
                         int classify, uint32_t* tileStates, bool seedTiles, int primaryTargetBlocks, int heavyTargetTiles, \
                         cudaStream_t stream);                                                                           \
-    void launch_shade(const DevFrame& fr, const FramePointers& fp, const BandView& band, const ActiveList& list,        \
-                      int gridBlocks, unsigned int* groupCounter, unsigned int firstSlot, cudaStream_t stream,          \
-                      int variant = 1);
+    int launch_shade(const DevFrame& fr, const FramePointers& fp, const BandView& band, const ActiveList& list,         \
+                     int gridBlocks, unsigned int* groupCounter, unsigned int firstSlot, cudaStream_t stream,           \
+                     int variant = 1, const McAovTargets* aov = nullptr);
 // Primary pass: per-tile jitter stream, camera rays, hit/miss classification, background
 // resolve of pixels no sample of which hits, work records for the rest.
 // classify == 0 puts every pixel on the work list (used for spp > 256 and for tests).
@@ -131,6 +135,7 @@ namespace counter {
 MCSKIN_HOT_KERNEL_LAUNCHERS
 }
 // Shading pass: full integrator for every sample of every listed pixel, ordered resolve.
+// aov: the AOV planes of the listed pixels too (a second, small kernel).  Returns the kernels launched.
 // Megakernel form of the shading pass over the listed pixels from `firstSlot` on.
 // variant 1: block-synchronous groups; variant 2: warp-autonomous groups with dynamic
 // distribution (groupCounter: a zeroed device counter; spp must be a power of two <= 32).

@@ -84,10 +84,11 @@ __device__ __forceinline__ bool enqueue_hit(const HitQueueView& q, unsigned int*
 // The 32 samples of a warp belong to 32 / spp neighbouring pixels, so the lanes that bounce do so together.
 constexpr int kPathOverflow = -2;  // top[path]: the queue was full; the path is redone in-thread (k_wf_overflow)
 
-template <bool BATCH>
+// AOV: also record every path's camera-ray hit (AovView::t / id) for the AOV planes.
+template <bool BATCH, bool AOV>
 __global__ void WF_HIT0_BOUNDS
-k_wf_trace(const DevFrame fr, const FramePointers fp_, const ActiveList list_, const WaveView wv_,
-           const BatchSlice* __restrict__ batch) {
+k_wf_trace(const DevFrame fr, const FramePointers fp_, const ActiveList list_, const WaveView wv_, const AovView aov_,
+           const AovView* __restrict__ aovBatch, const BatchSlice* __restrict__ batch) {
     __shared__ __align__(8) uint64_t stageBar;
     const FramePointers& fp = BATCH ? batch[blockIdx.y].fp : fp_;
     const ActiveList& list = BATCH ? batch[blockIdx.y].list : list_;
@@ -135,6 +136,11 @@ k_wf_trace(const DevFrame fr, const FramePointers fp_, const ActiveList list_, c
                 // pass does, measured slower here: the branch-free reject pass over all boxes is cheaper than
                 // the mask plus a bit loop when nearly every ray hits)
                 hit = closest_hit(sc, ray);
+                if (AOV) {
+                    const AovView& av = BATCH ? aovBatch[blockIdx.y] : aov_;
+                    av.t[p] = hit.t;
+                    av.id[p] = aov_id(hit);
+                }
                 if (fr.max_bounces < 0) {
                     // traceRay returns at once (depth 0 > maxBounces, raytracer.cpp:86-90); the tile
                     // renderer's re-test replaces misses by the gradient (tile_renderer.cpp:111-114)
@@ -465,10 +471,11 @@ __device__ __forceinline__ float4 fold_path(const WaveView& wv, size_t path) {
 
 // FAR: the form for images across a link (BandView::far_output); two instantiations, so that the streaming form keeps
 // its 32 registers (8 resident blocks: the kernel lives on loads in flight).
-template <bool BATCH, bool FAR>
+// AOV: the first lane of every pixel also folds the pixel's recorded camera-ray hits in sample order (store_aov).
+template <bool BATCH, bool FAR, bool AOV>
 __global__ void __launch_bounds__(kWfThreads)
 k_wf_resolve_warp(const DevFrame fr, const BandView band_, const ActiveList list_, const WaveView wv_, const int lgSpp,
-                  const BatchSlice* __restrict__ batch) {
+                  const AovView aov_, const AovView* __restrict__ aovBatch, const BatchSlice* __restrict__ batch) {
     const BandView band = hot_band(BATCH ? batch[blockIdx.y].band : band_);  // listed pixels lie in tiles the figure's rectangle touches
     const ActiveList& list = BATCH ? batch[blockIdx.y].list : list_;
     const WaveView& wv = BATCH ? batch[blockIdx.y].wave : wv_;
@@ -499,6 +506,13 @@ k_wf_resolve_warp(const DevFrame fr, const BandView band_, const ActiveList list
             resolveMask |= 1u << (l >> lgSpp);
         }
         warp_resolve(fr, band, stageW, lane, spp, lgSpp, colour, pixelIndex, resolveMask, outStage);
+        if (AOV && on && s == 0) {
+            const AovView& av = BATCH ? aovBatch[blockIdx.y] : aov_;
+            const size_t path0 = static_cast<size_t>(slot) * spp;
+            AovFold a;
+            for (int i = 0; i < spp; ++i) a.add(av.t[path0 + i], av.id[path0 + i]);
+            store_aov(fr, av.planes, pixelIndex, a);
+        }
     };
     if (!FAR) {
         // the image is this device's memory: rounds dealt to the warps of the grid in turn (the grid streams through the
@@ -536,10 +550,10 @@ k_wf_resolve_warp(const DevFrame fr, const BandView band_, const ActiveList list
 }
 
 // any spp: one thread sums a pixel's folded samples in order
-template <bool BATCH>
+template <bool BATCH, bool AOV>
 __global__ void __launch_bounds__(kWfThreads)
 k_wf_resolve_pixel(const DevFrame fr, const BandView band_, const ActiveList list_, const WaveView wv_,
-                   const BatchSlice* __restrict__ batch) {
+                   const AovView aov_, const AovView* __restrict__ aovBatch, const BatchSlice* __restrict__ batch) {
     const BandView band = hot_band(BATCH ? batch[blockIdx.y].band : band_);
     const ActiveList& list = BATCH ? batch[blockIdx.y].list : list_;
     const WaveView& wv = BATCH ? batch[blockIdx.y].wave : wv_;
@@ -554,6 +568,12 @@ k_wf_resolve_pixel(const DevFrame fr, const BandView band_, const ActiveList lis
         float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
         for (int s = 0; s < spp; ++s) acc = add4(acc, fold_path(wv, static_cast<size_t>(slot) * spp + s));
         store_pixel(band, sp.x, scale4(acc, fr.inv_spp));
+        if (AOV) {
+            const AovView& av = BATCH ? aovBatch[blockIdx.y] : aov_;
+            AovFold a;
+            for (int s = 0; s < spp; ++s) a.add(av.t[static_cast<size_t>(slot) * spp + s], av.id[static_cast<size_t>(slot) * spp + s]);
+            store_aov(fr, av.planes, sp.x, a);
+        }
     }
 }
 
@@ -588,14 +608,15 @@ constexpr int kQueueCounters = 4;
 }  // namespace
 
 int wavefront_max_hits_per_path(const DevFrame& fr) { return stack_levels_of(fr) + 1; }
-size_t wavefront_bytes_per_path(const DevFrame& fr) {
-    return sizeof(float4) + sizeof(int) + sizeof(float4) * stack_levels_of(fr);  // tail, top, bounce stack
+size_t wavefront_bytes_per_path(const DevFrame& fr, bool aov) {
+    // tail, top, bounce stack (+ the camera ray's hit distance and id)
+    return sizeof(float4) + sizeof(int) + sizeof(float4) * stack_levels_of(fr) + (aov ? sizeof(float) + sizeof(int) : 0);
 }
 size_t wavefront_bytes_per_entry() { return kEntryBytes; }
 size_t wavefront_fixed_bytes(const DevFrame&) { return 256 * 16 + sizeof(unsigned int) * kQueueCounters; }
 
 bool wavefront_carve(const DevFrame& fr, void* base, size_t bytes, unsigned int pathCapacity, unsigned int entryCapacity,
-                     int gridBlocks, WaveView* out) {
+                     int gridBlocks, WaveView* out, AovView* aov) {
     WaveView w{};
     w.pathCapacity = pathCapacity;
     w.slotCapacity = pathCapacity / static_cast<unsigned int>(fr.spp);
@@ -622,7 +643,13 @@ bool wavefront_carve(const DevFrame& fr, void* base, size_t bytes, unsigned int 
     w.stack = static_cast<float4*>(take(std::max<size_t>(16, cap * sizeof(float4) * w.levels)));
     // [0] hits in the queue (counts on beyond the capacity: overflow), [1] chunk counter of the soft-shadow kernel
     w.qCount = static_cast<unsigned int*>(take(sizeof(unsigned int) * kQueueCounters));
+    float* aovT = aov ? static_cast<float*>(take(cap * sizeof(float))) : nullptr;
+    int* aovId = aov ? static_cast<int*>(take(cap * sizeof(int))) : nullptr;
     if (off > bytes) return false;
+    if (aov) {
+        aov->t = aovT;
+        aov->id = aovId;
+    }
     *out = w;
     return true;
 }
@@ -633,8 +660,9 @@ void launch_batch_reset(const BatchSlice* batch, int nScenes, cudaStream_t strea
 
 void launch_wavefront(const DevFrame& fr, const FramePointers& fp, const BandView& band, const ActiveList& list,
                       const WaveView& wv, unsigned int* groupCounter, cudaStream_t stream, int* launches,
-                      const BatchSlice* batch, int nScenes) {
+                      const BatchSlice* batch, int nScenes, const AovView* aovView, const AovView* aovBatch) {
     int n = 0;
+    const AovView av = aovView ? *aovView : AovView{};
     const int grid = wv.gridBlocks;
     const unsigned int ny = batch ? static_cast<unsigned int>(nScenes) : 1u;
     const dim3 g(grid, ny);
@@ -654,7 +682,15 @@ void launch_wavefront(const DevFrame& fr, const FramePointers& fp, const BandVie
     // a batch's queue counters are zeroed by the caller (one kernel over all scenes)
     if (!batch) cudaMemsetAsync(wv.qCount, 0, sizeof(unsigned int) * kQueueCounters, stream);
     // every hit of every path, all bounce depths, into the one queue
-    MCSKIN_WF_LAUNCH(k_wf_trace, g, blob, fr, fp, list, wv);
+    const bool aov = batch ? aovBatch != nullptr : av.t != nullptr;
+    if (batch) {
+        if (aov) k_wf_trace<true, true><<<g, kWfThreads, blob, stream>>>(fr, fp, list, wv, av, aovBatch, batch);
+        else k_wf_trace<true, false><<<g, kWfThreads, blob, stream>>>(fr, fp, list, wv, av, aovBatch, batch);
+    } else {
+        if (aov) k_wf_trace<false, true><<<g, kWfThreads, blob, stream>>>(fr, fp, list, wv, av, aovBatch, batch);
+        else k_wf_trace<false, false><<<g, kWfThreads, blob, stream>>>(fr, fp, list, wv, av, aovBatch, batch);
+    }
+    ++n;
     if (fr.max_bounces >= 0) {
         if (wv.shadowMode == kShadowSoft) {
             // persistent blocks that claim chunks of 256 hits: no more of them than can be resident
@@ -679,18 +715,28 @@ void launch_wavefront(const DevFrame& fr, const FramePointers& fp, const BandVie
     const int lg = log2_pow2_le32(fr.spp);
     if (lg >= 0) {
         const bool farImage = !batch && band.far_output != 0;
-        if (batch) k_wf_resolve_warp<true, false><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, lg, batch);
-        else if (farImage) k_wf_resolve_warp<false, true><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, lg, batch);
-        else k_wf_resolve_warp<false, false><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, lg, batch);
+        if (aov) {
+            if (batch) k_wf_resolve_warp<true, false, true><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, lg, av, aovBatch, batch);
+            else if (farImage) k_wf_resolve_warp<false, true, true><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, lg, av, aovBatch, batch);
+            else k_wf_resolve_warp<false, false, true><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, lg, av, aovBatch, batch);
+        } else {
+            if (batch) k_wf_resolve_warp<true, false, false><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, lg, av, aovBatch, batch);
+            else if (farImage) k_wf_resolve_warp<false, true, false><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, lg, av, aovBatch, batch);
+            else k_wf_resolve_warp<false, false, false><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, lg, av, aovBatch, batch);
+        }
+        ++n;
+    } else {
+        if (batch && aov) k_wf_resolve_pixel<true, true><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, av, aovBatch, batch);
+        else if (batch) k_wf_resolve_pixel<true, false><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, av, aovBatch, batch);
+        else if (aov) k_wf_resolve_pixel<false, true><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, av, aovBatch, batch);
+        else k_wf_resolve_pixel<false, false><<<g, kWfThreads, 0, stream>>>(fr, band, list, wv, av, aovBatch, batch);
         ++n;
     }
-    else MCSKIN_WF_LAUNCH(k_wf_resolve_pixel, g, 0, fr, band, list, wv);
 #undef MCSKIN_WF_LAUNCH
     // pixels the queues could not take: megakernel, starting at the first slot beyond them
     // (never in a batch: its queues are sized for every pixel of a scene)
     if (!batch && wv.slotCapacity < list.capacity) {
-        MCSKIN_VARIANT_NS::launch_shade(fr, fp, band, list, grid, groupCounter, wv.slotCapacity, stream);  // (this build's)
-        ++n;
+        n += MCSKIN_VARIANT_NS::launch_shade(fr, fp, band, list, grid, groupCounter, wv.slotCapacity, stream, 1, aov ? &av.planes : nullptr);  // (this build's)
     }
     if (launches) *launches += n;
 }

@@ -58,6 +58,15 @@ struct WaveView {
     uint2* seedMemo;         // FreshStream::seed_memo's table (kSeedMemoEntries entries), or null
 };
 
+// The AOV planes of a frame (or of one scene of a batch) and the wavefront's per-path records of them: the camera ray's
+// closest hit, distance and McHit-style id (-1: miss), written by k_wf_trace and folded per pixel by the resolve kernels.
+// Kept apart from WaveView and BatchSlice: the batched kernels index a BatchSlice array, whose 256-byte stride is a shift.
+struct AovView {
+    McAovTargets planes;
+    float* t;
+    int* id;
+};
+
 enum : int {
     kShadowHard = 0,      // no soft shadows: one ray to the light centre, normalised normal (shade())
     kShadowSoft = 1,      // computeSoftShadow with 2 <= N <= 113 samples: seed + N rays per hit
@@ -74,29 +83,40 @@ struct BatchSlice {
     ActiveList list;
     WaveView wave;
 };
+static_assert(sizeof(BatchSlice) == 256, "a BatchSlice is indexed by blockIdx.y: keep its stride a power of two");
 
 // Storage: per path (terminal colour, stack height, bounce stack), per queue entry (hit record + lit counter).
-size_t wavefront_bytes_per_path(const DevFrame& fr);
+// aov: the frame writes AOV planes (8 more bytes per path).
+size_t wavefront_bytes_per_path(const DevFrame& fr, bool aov = false);
 size_t wavefront_bytes_per_entry();
 size_t wavefront_fixed_bytes(const DevFrame& fr);
 // Hits a path can put into the queue: bounce levels + 1.  A queue of pathCapacity times this cannot overflow.
 int wavefront_max_hits_per_path(const DevFrame& fr);
 // Carves the views out of one allocation of at least pathCapacity * wavefront_bytes_per_path +
 // entryCapacity * wavefront_bytes_per_entry + wavefront_fixed_bytes (+ 256 per array) bytes; false if too small.
+// aov (frames with AOV planes): also carves its per-path records (aov->t, aov->id).
 bool wavefront_carve(const DevFrame& fr, void* base, size_t bytes, unsigned int pathCapacity, unsigned int entryCapacity,
-                     int gridBlocks, WaveView* out);
+                     int gridBlocks, WaveView* out, AovView* aov = nullptr);
+
+// The AOV defaults (coverage 0, depth 0, tri_id -1) into every pixel of the band's tiles (of every scene of a batch), before
+// the primary pass; the shading pass then overwrites the pixels it resolves.  Only for bands with AOV planes.
+// aovBatch: the device array of a batch's per-scene AOV views (null: one frame, `planes`).
+void launch_aov_defaults(const DevFrame& fr, const BandView& band, const McAovTargets& planes, const AovView* aovBatch, int nScenes,
+                         cudaStream_t stream);
 
 // Shades every listed pixel (slots < wave.slotCapacity through the wavefront, the rest through the
 // megakernel) and writes the band image.  groupCounter: zeroed device counter.
 // batch / nScenes: device array of per-scene slices and its length (launches get gridDim.y = nScenes);
 // every slice must have slotCapacity >= its list's capacity (no megakernel overflow in batches).
+// aov / aovBatch: the frame's AOV view, or the device array of a batch's per-scene views (null: no AOV planes).
 // launch_primary_batch: the primary pass over the scenes of a batch (pixel-per-lane kernels only): returns false if the
 // frame description needs one of the other primary kernels, which have no batched form.
 // (declared for both builds of the kernels: dev_types.cuh)
 #define MCSKIN_HOT_WAVEFRONT_LAUNCHERS                                                                                   \
     void launch_wavefront(const DevFrame& fr, const FramePointers& fp, const BandView& band, const ActiveList& list,    \
                           const WaveView& wave, unsigned int* groupCounter, cudaStream_t stream, int* launches,         \
-                          const BatchSlice* batch = nullptr, int nScenes = 1);                                          \
+                          const BatchSlice* batch = nullptr, int nScenes = 1, const AovView* aov = nullptr,             \
+                          const AovView* aovBatch = nullptr);                                                          \
     void launch_batch_reset(const BatchSlice* batch, int nScenes, cudaStream_t stream);                                 \
     bool launch_primary_batch(const DevFrame& fr, const BandView& band, uint32_t* tileStates, bool seedTiles,           \
                               const BatchSlice* batch, int nScenes, unsigned int blobBytes, int primaryTargetBlocks,    \

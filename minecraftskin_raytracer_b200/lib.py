@@ -40,7 +40,7 @@ EXPORTS = [
     "mcskin_cuda_host_register", "mcskin_cuda_host_unregister", "mcskin_cuda_render_batch_multi",
     "mcskin_cuda_enable_peer_access", "mcskin_cuda_context_render_scene_tiles",
     "mcskin_cuda_context_debug_block_times", "mcskin_cuda_context_render_skin_batch",
-    "mcskin_skin_layout",
+    "mcskin_skin_layout", "mcskin_cuda_render_aovs", "mcskin_cuda_context_set_aov_targets",
 ]
 
 
@@ -207,6 +207,29 @@ def render(scene, cfg: McConfig, device: int = 0, want_f32: bool = True, want_u8
     return f32, u8, {k: getattr(stats, k) for k, _ in McRenderStats._fields_}
 
 
+def render_aovs(scene, cfg: McConfig, device: int = 0, want_u8: bool = False):
+    """mcskin_cuda_render_aovs: the frame of `render` plus its AOV planes.  Returns (f32 [H, W, 4], u8 [H, W, 4] | None,
+    {"coverage": float32 [H, W], "depth": float32 [H, W], "tri_id": int32 [H, W]}, stats dict)."""
+    h, w = max(cfg.height, 0), max(cfg.width, 0)
+    f32 = np.empty((h, w, 4), dtype=np.float32)
+    u8 = np.empty((h, w, 4), dtype=np.uint8) if want_u8 else None
+    n_tiles = len(generate_tiles(cfg.width, cfg.height, cfg.tile_size)) if (w and h) else 0
+    if n_tiles == 0 and f32.size:  # nothing is rendered: Image(w,h) pixels stay (0,0,0,1) (image.h:15, color.h:8)
+        f32[...] = 0
+        f32[..., 3] = 1
+        if u8 is not None:
+            u8[...] = 0
+            u8[..., 3] = 255
+    planes = {"coverage": np.empty((h, w), dtype=np.float32), "depth": np.empty((h, w), dtype=np.float32),
+              "tri_id": np.empty((h, w), dtype=np.int32)}
+    targets = _abi.McAovTargets(planes["coverage"].ctypes.data, planes["depth"].ctypes.data, planes["tri_id"].ctypes.data)
+    stats = McRenderStats()
+    cs = scene.as_c() if isinstance(scene, FlatScene) else scene
+    _check(_lib.mcskin_cuda_render_aovs(C.byref(cs), C.byref(cfg), C.c_int32(device), _ptr(f32, C.c_float),
+                                        None if u8 is None else _ptr(u8, C.c_uint8), C.byref(targets), C.byref(stats)))
+    return f32, u8, planes, {k: getattr(stats, k) for k, _ in McRenderStats._fields_}
+
+
 def render_batch_multi(scenes: list[FlatScene], cfg: McConfig, n_devices: int, want_f32: bool = True, want_u8: bool = False):
     """mcskin_cuda_render_batch_multi: a batch of skins, host scenes in, host images out, skin i on device i % n_devices.
     Returns (f32 [n, H, W, 4] | None, u8 [n, H, W, 4] | None)."""
@@ -331,6 +354,12 @@ class Context:
 
     def set_option(self, name: str, value: int):
         _check(_lib.mcskin_cuda_context_set_option(self._h, name.encode(), C.c_int64(value)))
+
+    def set_aov_targets(self, coverage: int = 0, depth: int = 0, tri_id: int = 0):
+        """AOV planes for the following render calls: raw device addresses of float32 / float32 / int32 planes laid out
+        like the colour image of each call (0: that plane is not written; all 0 switches them off)."""
+        t = _abi.McAovTargets(coverage or None, depth or None, tri_id or None)
+        _check(_lib.mcskin_cuda_context_set_aov_targets(self._h, C.byref(t)))
 
     def set_scene(self, scene: FlatScene, cfg: McConfig):
         cs = scene.as_c()
