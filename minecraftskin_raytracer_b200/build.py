@@ -18,7 +18,7 @@ LIB_PATH = LIB_DIR / "libmcskin_cuda.so"
 # kernels_plain.cu / wavefront_plain.cu: the same kernels built without pose code (csrc/dev_types.cuh)
 # kernels_counter.cu / wavefront_counter.cu: the general kernels with counter-based random streams (McConfig::rng_mode 1)
 CUDA_SOURCES = ["kernels.cu", "wavefront.cu", "kernels_plain.cu", "wavefront_plain.cu", "kernels_counter.cu",
-                "wavefront_counter.cu", "capi.cu"]
+                "wavefront_counter.cu", "capi.cu", "context.cu", "frame.cu", "host_out.cu", "batch.cu"]
 HOST_SOURCES = ["host_prep.cpp", "skin_scene.cpp", "host_copy.cpp"]
 
 # --fmad=false: the geometry chain must round like the x86-64 reference build (no FMA);

@@ -1321,16 +1321,6 @@ static size_t pix_smem_limit() {
     return optIn.limit(fns, static_cast<int>(sizeof(fns) / sizeof(fns[0])));
 }
 
-// Engine states the pixel-per-lane primary kernels keep per tile for a launch of nTiles tiles x nScenes scenes: 1 (the
-// seed) when no tile is split over blocks, else one per round of 256 pixels.  The host sizes tileStates with it.
-int primary_states_per_tile(const DevFrame& fr, int nTiles, int nScenes, int primaryTargetBlocks, int heavyTargetTiles) {
-    if (nTiles <= 0 || fr.draws_per_sample <= 0) return 1;
-    const int roundsPerTile = (fr.tile_size * fr.tile_size + kBlockThreads - 1) / kBlockThreads;
-    const long long allTiles = static_cast<long long>(nTiles) * std::max(1, nScenes);
-    const bool split = primaryTargetBlocks > allTiles || heavyTargetTiles > allTiles;
-    return split && roundsPerTile > 1 ? roundsPerTile : 1;
-}
-
 // The pixel-per-lane primary kernels over one scene (batch == nullptr) or the scenes of a batch.
 static void launch_primary_pix(const DevFrame& fr, const FramePointers& fp, const BandView& band, const ActiveList& list,
                                uint32_t* tileStates, bool seedTiles, int primaryTargetBlocks, int heavyTargetTiles,
@@ -1350,7 +1340,7 @@ static void launch_primary_pix(const DevFrame& fr, const FramePointers& fp, cons
     while (roundsPerTile % partsHeavy) --partsHeavy;
     TileOrder order = make_tile_order(fr, band, partsHeavy, parts);
     // split tiles start every block at its own round of the tile's stream (k_tile_rounds)
-    const int statesPerTile = MCSKIN_VARIANT_NS::primary_states_per_tile(fr, nTiles, batch ? nScenes : 1, primaryTargetBlocks, heavyTargetTiles);
+    const int statesPerTile = primary_states_per_tile(fr, nTiles, batch ? nScenes : 1, primaryTargetBlocks, heavyTargetTiles);
     order.round_states = statesPerTile > 1 ? statesPerTile : 0;
     // the seeded engines depend on the tile geometry only: one set serves every scene of a batch
     if (fr.draws_per_sample > 0 && seedTiles) {

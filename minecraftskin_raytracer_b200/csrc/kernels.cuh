@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
 #include <mutex>
 
 #include "dev_types.cuh"
@@ -140,14 +141,15 @@ MCSKIN_HOT_KERNEL_LAUNCHERS
 // variant 1: block-synchronous groups; variant 2: warp-autonomous groups with dynamic
 // distribution (groupCounter: a zeroed device counter; spp must be a power of two <= 32).
 
-// Engine states per tile the primary pass keeps for such a launch (1 = the seed only; more: one per round of 256
-// pixels, for tiles split over blocks): tileStates must hold nTiles * this * 624 words.
-int primary_states_per_tile(const DevFrame& fr, int nTiles, int nScenes, int primaryTargetBlocks, int heavyTargetTiles);
-namespace plain {
-int primary_states_per_tile(const DevFrame& fr, int nTiles, int nScenes, int primaryTargetBlocks, int heavyTargetTiles);
-}
-namespace counter {
-int primary_states_per_tile(const DevFrame& fr, int nTiles, int nScenes, int primaryTargetBlocks, int heavyTargetTiles);
+// Engine states the pixel-per-lane primary kernels keep per tile for a launch of nTiles tiles x nScenes scenes: 1 (the
+// seed) when no tile is split over blocks, else one per round of 256 pixels.  tileStates must hold nTiles * this * 624
+// words.  (Host arithmetic, the same for every build of the kernels.)
+inline int primary_states_per_tile(const DevFrame& fr, int nTiles, int nScenes, int primaryTargetBlocks, int heavyTargetTiles) {
+    if (nTiles <= 0 || fr.draws_per_sample <= 0) return 1;
+    const int roundsPerTile = (fr.tile_size * fr.tile_size + kBlockThreads - 1) / kBlockThreads;
+    const long long allTiles = static_cast<long long>(nTiles) * std::max(1, nScenes);
+    const bool split = primaryTargetBlocks > allTiles || heavyTargetTiles > allTiles;
+    return split && roundsPerTile > 1 ? roundsPerTile : 1;
 }
 
 // Single-query views of the same device code (all pointers are device memory).

@@ -20,7 +20,7 @@ import os
 # MCSKIN_LIB selects an alternative build of the same library (kernel tuning experiments)
 LIB_PATH = Path(os.environ.get("MCSKIN_LIB") or (Path(__file__).resolve().parent / "_lib" / "libmcskin_cuda.so"))
 
-# streams a frame's tile rows are dealt to by default (McContext::frameLanes in csrc/capi.cu)
+# streams a frame's tile rows are dealt to by default (McOptions::frameLanes in csrc/capi_internal.hpp)
 DEFAULT_FRAME_LANES = 2
 
 # every symbol include/mcskin_cuda.h declares
