@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define MCSKIN_ABI_VERSION 2
+#define MCSKIN_ABI_VERSION 3
 
 enum {
     MC_OK = 0,
@@ -175,15 +175,28 @@ int32_t mcskin_cuda_render(const McScene* scene, const McConfig* cfg, int32_t de
  *   coverage : (float)n * (1.0f / (float)spp)
  *   depth    : the hit distances h_s.t of the hitting samples summed left to right from 0.0f, divided by (float)n;
  *              0.0f when n == 0
- *   tri_id   : box*12 + face*2 of the first hitting sample (the McHit / mcskin_cuda_aov convention); -1 when n == 0 */
+ *   tri_id   : box*12 + face*2 of the first hitting sample (the McHit / mcskin_cuda_aov convention); -1 when n == 0
+ * The guide planes a denoiser or compositor takes next to the colour, 3 and 4 floats per pixel (pixel i at 3*i, 4*i):
+ *   normal   : McHit.normal of the hitting samples (the outer-layer exit-face flip included, posed boxes back-transformed),
+ *              each component summed left to right from 0.0f (so a -0 component reads +0) and divided by (float)n; not
+ *              renormalised.  (0, 0, 0) when n == 0
+ *   albedo   : the same fold over McHit.tex_color (magenta for a null texture, (0, 0, 0, 1) for an empty region);
+ *              (0, 0, 0, 0) when n == 0
+ * A hit never has a texel of alpha 0: such texels are passed through, and the outer-layer exit face is taken only when
+ * its alpha is > 0.  So when no texel alpha is negative (every skin built from an 8-bit atlas), albedo's alpha is > 0
+ * exactly where tri_id >= 0.
+ * (normal and albedo were appended in ABI version 3.) */
 typedef struct McAovTargets {
     float* coverage;
     float* depth;
     int32_t* tri_id;
+    float* normal;
+    float* albedo;
 } McAovTargets;
 
 /* mcskin_cuda_render with AOV planes: the same colour bytes, and the planes `aov` asks for (host memory, width*height
- * values each; aov may be NULL).  A frame with no tiles leaves the defaults (0, 0, -1) in every requested plane. */
+ * values each, 3 and 4 times that for normal and albedo; aov may be NULL).  A frame with no tiles leaves the defaults
+ * (0, 0, -1, zeros, zeros) in every requested plane. */
 int32_t mcskin_cuda_render_aovs(const McScene* scene, const McConfig* cfg, int32_t device,
                                 float* out_rgba_f32, uint8_t* out_rgba_u8, const McAovTargets* aov,
                                 McRenderStats* stats);
@@ -282,7 +295,7 @@ int32_t mcskin_cuda_context_debug_block_times(McContext* ctx, uint64_t* out, int
 /* AOV planes for the context's later render calls: d_targets holds DEVICE-addressable pointers (copied; NULL, or all
  * members NULL, switches the planes off).  render_bands, render_rows_into_frame, render_tiles_into_frame, render_batch and
  * render_skin_batch then write every plane that is set for every pixel they render, at the colour image's index (image i
- * of a batch at offset i*width*height); frame lanes inherit the targets.  render_scene_tiles fails with MC_ERR_INVALID
+ * of a batch at offset i*width*height, times 3 for normal and 4 for albedo); frame lanes inherit the targets.  render_scene_tiles fails with MC_ERR_INVALID
  * while targets are set. */
 int32_t mcskin_cuda_context_set_aov_targets(McContext* ctx, const McAovTargets* d_targets);
 /* Blocks until the context's work is done, fills stats of the last render. */

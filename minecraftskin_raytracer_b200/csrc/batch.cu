@@ -67,7 +67,7 @@ int render_batch_grouped(McContext* ctx, const McScene* scenes, const SkinBatchS
     const size_t entries = paths * static_cast<size_t>(wavefront_max_hits_per_path(f0));  // cannot overflow
     if (entries > 0xffffff00u) return MC_OK;
     const bool aov = aov_on(ctx);
-    const size_t waveBytes = (paths * wavefront_bytes_per_path(f0, aov) + entries * wavefront_bytes_per_entry() +
+    const size_t waveBytes = (paths * wavefront_bytes_per_path(f0, aov, aov_guides(ctx->aov)) + entries * wavefront_bytes_per_entry() +
                               wavefront_fixed_bytes(f0) + 16 * 256 + 255) & ~size_t(255);
     const size_t perScene = waveBytes + recordBytes + slotCap * sizeof(uint2);
     int G = std::min<int>(ctx->batchGroup, nScenes);
@@ -209,7 +209,7 @@ int render_batch_grouped(McContext* ctx, const McScene* scenes, const SkinBatchS
                 // few blocks per scene: a launch has gridDim.y scenes to fill the machine with
                 const int gridX = std::max(2, (ctx->smCount * ctx->shadeBlocksPerSm + nC - 1) / nC);
                 if (!wavefront_carve(pf.frame, static_cast<unsigned char*>(ctx->batchWave.p) + static_cast<size_t>(i) * waveBytes,
-                                     waveBytes, static_cast<unsigned int>(paths), static_cast<unsigned int>(entries), gridX, &sl.wave, aov ? &av : nullptr))
+                                     waveBytes, static_cast<unsigned int>(paths), static_cast<unsigned int>(entries), gridX, &sl.wave, aov ? &av.planes : nullptr))
                     return MC_OK;  // (cannot happen: the sizes depend on the config only) frame-by-frame path instead
                 sl.wave.seedMemo = batchSeedMemo;
                 stageAovs[sliceAt] = av;

@@ -155,6 +155,7 @@ struct McContext : McOptions {
         int nTiles, nHeavy;
         const void *hotF32, *hotU8;
         const void *aovCoverage, *aovDepth, *aovTriId;  // a graph with AOV stores is never replayed without them, or vice versa
+        const void *aovNormal, *aovAlbedo;
         long long optionBits[kOptionCount];             // the launch options (0 for the others)
         unsigned long long allocEpoch;
         bool operator==(const GraphKey& o) const { return std::memcmp(this, &o, sizeof(GraphKey)) == 0; }
@@ -209,13 +210,15 @@ constexpr KernelBuild kCounterBuild{&counter::launch_primary, &counter::launch_s
 
 inline const KernelBuild& kernels_for(const DevFrame& f) { return f.rng_mode ? kCounterBuild : (f.any_rotated ? kGeneralBuild : kPlainBuild); }
 
-inline bool aov_on(const McContext* ctx) { return ctx->aov.coverage || ctx->aov.depth || ctx->aov.tri_id; }
+inline bool aov_on(const McContext* ctx) { return aov_any(&ctx->aov); }
 // the planes of the image that starts `pixels` pixels into the targets (image i of a batch)
 inline McAovTargets aov_at(const McAovTargets& a, size_t pixels) {
     McAovTargets r{};
     r.coverage = a.coverage ? a.coverage + pixels : nullptr;
     r.depth = a.depth ? a.depth + pixels : nullptr;
     r.tri_id = a.tri_id ? a.tri_id + pixels : nullptr;
+    r.normal = a.normal ? a.normal + 3 * pixels : nullptr;
+    r.albedo = a.albedo ? a.albedo + 4 * pixels : nullptr;
     return r;
 }
 

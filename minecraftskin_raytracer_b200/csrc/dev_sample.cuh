@@ -85,6 +85,33 @@ __device__ __forceinline__ void store_aov(const DevFrame& fr, const McAovTargets
     if (planes.depth) planes.depth[index] = a.n > 0 ? a.tsum / static_cast<float>(a.n) : 0.0f;
     if (planes.tri_id) planes.tri_id[index] = a.id;
 }
+// The guide planes of a pixel (McAovTargets::normal, ::albedo): McHit.normal and McHit.tex_color of its hitting samples,
+// summed left to right from 0 in sample order.  store_guides divides by the hit count n of the pixel's AovFold (zeros
+// when n == 0) and writes pixel `index` at 3 * index and 4 * index.
+struct GuideFold {
+    float nx = 0.0f, ny = 0.0f, nz = 0.0f;
+    float r = 0.0f, g = 0.0f, b = 0.0f, a = 0.0f;
+    __device__ __forceinline__ void add(float4 n, float4 c) {
+        nx += n.x; ny += n.y; nz += n.z;
+        r += c.x; g += c.y; b += c.z; a += c.w;
+    }
+};
+__device__ __forceinline__ void store_guides(const McAovTargets& planes, unsigned int index, int n, const GuideFold& f) {
+    const float fn = static_cast<float>(n);
+    if (planes.normal) {
+        float* o = planes.normal + 3 * static_cast<size_t>(index);
+        o[0] = n > 0 ? f.nx / fn : 0.0f;
+        o[1] = n > 0 ? f.ny / fn : 0.0f;
+        o[2] = n > 0 ? f.nz / fn : 0.0f;
+    }
+    if (planes.albedo) {
+        float* o = planes.albedo + 4 * static_cast<size_t>(index);
+        o[0] = n > 0 ? f.r / fn : 0.0f;
+        o[1] = n > 0 ? f.g / fn : 0.0f;
+        o[2] = n > 0 ? f.b / fn : 0.0f;
+        o[3] = n > 0 ? f.a / fn : 0.0f;
+    }
+}
 
 __device__ __forceinline__ float4 add4(float4 a, float4 b) {
     return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);

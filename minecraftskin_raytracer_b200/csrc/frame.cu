@@ -123,7 +123,7 @@ BandPlan plan_band(const DevFrame& f, const BandSpec& spec, const McContext& ctx
     // less than 1.25 entries per path; paths whose hits do not fit are redone in-thread), then the number of
     // paths does (pixels beyond them are shaded by the megakernel).
     if (ctx.shadeMode == 0) {
-        const size_t perPath = wavefront_bytes_per_path(f, aov_on(&ctx)), perEntry = wavefront_bytes_per_entry();
+        const size_t perPath = wavefront_bytes_per_path(f, aov_on(&ctx), aov_guides(ctx.aov)), perEntry = wavefront_bytes_per_entry();
         const size_t hitsMax = static_cast<size_t>(wavefront_max_hits_per_path(f));
         const size_t budget = static_cast<size_t>(ctx.waveBudgetBytes);
         const size_t worstPaths = p.slotCap * static_cast<size_t>(f.spp);
@@ -192,7 +192,7 @@ int render_bands_lane(McContext* ctx, const McContext* scn, const BandSpec& spec
         CU_TRY(ctx->wave.reserve(plan.waveBytes));
         if (!wavefront_carve(f, ctx->wave.p, ctx->wave.cap, static_cast<unsigned int>(plan.wavePaths),
                              static_cast<unsigned int>(plan.waveEntries), ctx->smCount * ctx->shadeBlocksPerSm, &wave,
-                             aov ? &aovView : nullptr))
+                             aov ? &ctx->aov : nullptr))
             return fail(MC_ERR_CUDA, "wavefront buffer carve failed");
         wave.softGrid = ctx->smCount * ctx->softBlocksPerSm;
         wave.seedMemo = static_cast<uint2*>(scn->seedMemo.p);  // (render_bands has seen to it; the lanes of a frame share it)
@@ -383,6 +383,7 @@ int render_bands(McContext* ctx, int first, int stride, float4* outF32, uchar4* 
         key.first = first; key.stride = stride; key.lanes = L * 2 + (frameLayout ? 1 : 0);
         key.hotF32 = hotF32; key.hotU8 = hotU8;
         key.aovCoverage = ctx->aov.coverage; key.aovDepth = ctx->aov.depth; key.aovTriId = ctx->aov.tri_id;
+        key.aovNormal = ctx->aov.normal; key.aovAlbedo = ctx->aov.albedo;
         if (tiles) {
             key.tileMap = tiles->map; key.mapVersion = tiles->mapVersion; key.nTiles = tiles->nTiles; key.nHeavy = tiles->nHeavy;
         }

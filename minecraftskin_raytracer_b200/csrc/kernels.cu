@@ -1066,7 +1066,9 @@ k_aov_defaults(const DevFrame fr, const BandView band, const McAovTargets planes
     const int nPix = tg.w * tg.h;
     for (int q = threadIdx.x; q < nPix; q += kBlockThreads) {
         const int ly = q / tg.w, lx = q - ly * tg.w;
-        store_aov(fr, planes, static_cast<unsigned int>(tg.bandRow0 + ly) * static_cast<unsigned int>(fr.width) + (tg.x + lx), AovFold{});
+        const unsigned int index = static_cast<unsigned int>(tg.bandRow0 + ly) * static_cast<unsigned int>(fr.width) + (tg.x + lx);
+        store_aov(fr, planes, index, AovFold{});
+        store_guides(planes, index, 0, GuideFold{});
     }
 }
 
@@ -1080,11 +1082,13 @@ k_aov_listed(const DevFrame fr, const FramePointers fp, const ActiveList list, c
     if (count > list.capacity) count = list.capacity;
     const SceneView sc = scene_view(fp.blob, fp.texels, fr);
     const int spp = fr.spp, dps = fr.draws_per_sample;
+    const bool guides = aov_guides(planes);
     for (unsigned int slot = firstSlot + blockIdx.x * kBlockThreads + threadIdx.x; slot < count; slot += gridDim.x * kBlockThreads) {
         const uint2 sp = list.slot_pixel[slot];
         if (sp.x == kUnusedSlot) continue;
         const int px = static_cast<int>(sp.y & 0xffffu), py = static_cast<int>(sp.y >> 16);
         AovFold a;
+        GuideFold g;
         for (int s = 0; s < spp; ++s) {
             float d0 = 0.0f, d1 = 0.0f, d2 = 0.0f, d3 = 0.0f;
             const float* rec = list.records + (static_cast<size_t>(slot) * spp + s) * dps;
@@ -1100,8 +1104,13 @@ k_aov_listed(const DevFrame fr, const FramePointers fp, const ActiveList list, c
             sample_uv(fr, px, py, sd, &u, &v);
             const Hit h = closest_hit(sc, primary_ray(fr, u, v, sd));
             a.add(h.t, aov_id(h));
+            if (guides && h.box >= 0) {
+                const V3 n = hit_normal(sc, h);
+                g.add(make_float4(n.x, n.y, n.z, 0.0f), hit_texel(sc, h));
+            }
         }
         store_aov(fr, planes, sp.x, a);
+        if (guides) store_guides(planes, sp.x, a.n, g);
     }
 }
 

@@ -92,7 +92,11 @@ __host__ __device__ inline int band_tile_count(const BandView& band, int tilesX)
 // AOV planes (McAovTargets, device pointers) travel next to a BandView, indexed like its out_f32: the launchers pick the
 // AOV instantiations of the shading kernels when any plane is set, and the kernels of frames without run as before.
 // (Not members of BandView: the batched primary kernels copy a scene's BandView, and a larger one costs them registers.)
-__host__ __device__ inline bool aov_any(const McAovTargets* a) { return a && (a->coverage || a->depth || a->tri_id); }
+__host__ __device__ inline bool aov_any(const McAovTargets* a) {
+    return a && (a->coverage || a->depth || a->tri_id || a->normal || a->albedo);
+}
+// the guide planes (normal, albedo): they need the camera ray's normal and texel colour as well as its distance and id
+__host__ __device__ inline bool aov_guides(const McAovTargets& a) { return a.normal || a.albedo; }
 
 // Work list produced by the primary pass for the shading pass.
 struct ActiveList {

@@ -84,7 +84,8 @@ __device__ __forceinline__ bool enqueue_hit(const HitQueueView& q, unsigned int*
 // The 32 samples of a warp belong to 32 / spp neighbouring pixels, so the lanes that bounce do so together.
 constexpr int kPathOverflow = -2;  // top[path]: the queue was full; the path is redone in-thread (k_wf_overflow)
 
-// AOV: also record every path's camera-ray hit (AovView::t / id) for the AOV planes.
+// AOV: also record every path's camera-ray hit for the AOV planes (aov_records; the normal and texel colour only when the
+// frame has a guide plane).
 template <bool BATCH, bool AOV>
 __global__ void WF_HIT0_BOUNDS
 k_wf_trace(const DevFrame fr, const FramePointers fp_, const ActiveList list_, const WaveView wv_, const AovView aov_,
@@ -138,8 +139,14 @@ k_wf_trace(const DevFrame fr, const FramePointers fp_, const ActiveList list_, c
                 hit = closest_hit(sc, ray);
                 if (AOV) {
                     const AovView& av = BATCH ? aovBatch[blockIdx.y] : aov_;
-                    av.t[p] = hit.t;
-                    av.id[p] = aov_id(hit);
+                    const AovRecords rec = aov_records(wv);
+                    rec.t[p] = hit.t;
+                    rec.id[p] = aov_id(hit);
+                    if (aov_guides(av.planes) && hit.box >= 0) {
+                        const V3 n = hit_normal(sc, hit);
+                        rec.normal[p] = make_float4(n.x, n.y, n.z, 0.0f);
+                        rec.albedo[p] = hit_texel(sc, hit);
+                    }
                 }
                 if (fr.max_bounces < 0) {
                     // traceRay returns at once (depth 0 > maxBounces, raytracer.cpp:86-90); the tile
@@ -469,9 +476,23 @@ __device__ __forceinline__ float4 fold_path(const WaveView& wv, size_t path) {
     return c;
 }
 
+// The AOV planes of the pixel whose spp paths start at path0, from the paths' records (k_wf_trace), in sample order.
+__device__ __forceinline__ void fold_aov(const DevFrame& fr, const McAovTargets& planes, const AovRecords& rec, size_t path0,
+                                         int spp, unsigned int pixelIndex) {
+    AovFold a;
+    for (int i = 0; i < spp; ++i) a.add(rec.t[path0 + i], rec.id[path0 + i]);
+    store_aov(fr, planes, pixelIndex, a);
+    if (!aov_guides(planes)) return;
+    GuideFold g;
+    for (int i = 0; i < spp; ++i)
+        if (rec.id[path0 + i] >= 0) g.add(rec.normal[path0 + i], rec.albedo[path0 + i]);
+    store_guides(planes, pixelIndex, a.n, g);
+}
+
 // FAR: the form for images across a link (BandView::far_output); two instantiations, so that the streaming form keeps
 // its 32 registers (8 resident blocks: the kernel lives on loads in flight).
-// AOV: the first lane of every pixel also folds the pixel's recorded camera-ray hits in sample order (store_aov).
+// AOV: the first lane of every pixel also folds the pixel's recorded camera-ray hits in sample order (store_aov,
+// store_guides).
 template <bool BATCH, bool FAR, bool AOV>
 __global__ void __launch_bounds__(kWfThreads)
 k_wf_resolve_warp(const DevFrame fr, const BandView band_, const ActiveList list_, const WaveView wv_, const int lgSpp,
@@ -508,10 +529,7 @@ k_wf_resolve_warp(const DevFrame fr, const BandView band_, const ActiveList list
         warp_resolve(fr, band, stageW, lane, spp, lgSpp, colour, pixelIndex, resolveMask, outStage);
         if (AOV && on && s == 0) {
             const AovView& av = BATCH ? aovBatch[blockIdx.y] : aov_;
-            const size_t path0 = static_cast<size_t>(slot) * spp;
-            AovFold a;
-            for (int i = 0; i < spp; ++i) a.add(av.t[path0 + i], av.id[path0 + i]);
-            store_aov(fr, av.planes, pixelIndex, a);
+            fold_aov(fr, av.planes, aov_records(wv), static_cast<size_t>(slot) * spp, spp, pixelIndex);
         }
     };
     if (!FAR) {
@@ -570,9 +588,7 @@ k_wf_resolve_pixel(const DevFrame fr, const BandView band_, const ActiveList lis
         store_pixel(band, sp.x, scale4(acc, fr.inv_spp));
         if (AOV) {
             const AovView& av = BATCH ? aovBatch[blockIdx.y] : aov_;
-            AovFold a;
-            for (int s = 0; s < spp; ++s) a.add(av.t[static_cast<size_t>(slot) * spp + s], av.id[static_cast<size_t>(slot) * spp + s]);
-            store_aov(fr, av.planes, sp.x, a);
+            fold_aov(fr, av.planes, aov_records(wv), static_cast<size_t>(slot) * spp, spp, sp.x);
         }
     }
 }
@@ -608,15 +624,16 @@ constexpr int kQueueCounters = 4;
 }  // namespace
 
 int wavefront_max_hits_per_path(const DevFrame& fr) { return stack_levels_of(fr) + 1; }
-size_t wavefront_bytes_per_path(const DevFrame& fr, bool aov) {
-    // tail, top, bounce stack (+ the camera ray's hit distance and id)
-    return sizeof(float4) + sizeof(int) + sizeof(float4) * stack_levels_of(fr) + (aov ? sizeof(float) + sizeof(int) : 0);
+size_t wavefront_bytes_per_path(const DevFrame& fr, bool aov, bool guides) {
+    // tail, top, bounce stack (+ the camera ray's hit distance and id, + its normal and texel colour)
+    return sizeof(float4) + sizeof(int) + sizeof(float4) * stack_levels_of(fr) + (aov ? sizeof(float) + sizeof(int) : 0) +
+           (aov && guides ? 2 * sizeof(float4) : 0);
 }
 size_t wavefront_bytes_per_entry() { return kEntryBytes; }
 size_t wavefront_fixed_bytes(const DevFrame&) { return 256 * 16 + sizeof(unsigned int) * kQueueCounters; }
 
 bool wavefront_carve(const DevFrame& fr, void* base, size_t bytes, unsigned int pathCapacity, unsigned int entryCapacity,
-                     int gridBlocks, WaveView* out, AovView* aov) {
+                     int gridBlocks, WaveView* out, const McAovTargets* aov) {
     WaveView w{};
     w.pathCapacity = pathCapacity;
     w.slotCapacity = pathCapacity / static_cast<unsigned int>(fr.spp);
@@ -643,13 +660,15 @@ bool wavefront_carve(const DevFrame& fr, void* base, size_t bytes, unsigned int 
     w.stack = static_cast<float4*>(take(std::max<size_t>(16, cap * sizeof(float4) * w.levels)));
     // [0] hits in the queue (counts on beyond the capacity: overflow), [1] chunk counter of the soft-shadow kernel
     w.qCount = static_cast<unsigned int*>(take(sizeof(unsigned int) * kQueueCounters));
-    float* aovT = aov ? static_cast<float*>(take(cap * sizeof(float))) : nullptr;
-    int* aovId = aov ? static_cast<int*>(take(cap * sizeof(int))) : nullptr;
-    if (off > bytes) return false;
-    if (aov) {
-        aov->t = aovT;
-        aov->id = aovId;
+    if (aov) {  // in aov_records' order, right after the counters
+        if (take(cap * sizeof(float)) != aov_records(w).t) return false;
+        take(cap * sizeof(int));
+        if (aov_guides(*aov)) {
+            take(cap * sizeof(float4));
+            take(cap * sizeof(float4));
+        }
     }
+    if (off > bytes) return false;
     *out = w;
     return true;
 }
@@ -682,7 +701,7 @@ void launch_wavefront(const DevFrame& fr, const FramePointers& fp, const BandVie
     // a batch's queue counters are zeroed by the caller (one kernel over all scenes)
     if (!batch) cudaMemsetAsync(wv.qCount, 0, sizeof(unsigned int) * kQueueCounters, stream);
     // every hit of every path, all bounce depths, into the one queue
-    const bool aov = batch ? aovBatch != nullptr : av.t != nullptr;
+    const bool aov = batch ? aovBatch != nullptr : aov_any(&av.planes);
     if (batch) {
         if (aov) k_wf_trace<true, true><<<g, kWfThreads, blob, stream>>>(fr, fp, list, wv, av, aovBatch, batch);
         else k_wf_trace<true, false><<<g, kWfThreads, blob, stream>>>(fr, fp, list, wv, av, aovBatch, batch);

@@ -58,14 +58,35 @@ struct WaveView {
     uint2* seedMemo;         // FreshStream::seed_memo's table (kSeedMemoEntries entries), or null
 };
 
-// The AOV planes of a frame (or of one scene of a batch) and the wavefront's per-path records of them: the camera ray's
-// closest hit, distance and McHit-style id (-1: miss), written by k_wf_trace and folded per pixel by the resolve kernels.
-// Kept apart from WaveView and BatchSlice: the batched kernels index a BatchSlice array, whose 256-byte stride is a shift.
+// The AOV planes of a frame (or of one scene of a batch).  Kept apart from WaveView and BatchSlice: the batched kernels
+// index a BatchSlice array, whose 256-byte stride is a shift.  The wavefront's per-path records of the planes lie in
+// the WaveView's buffer (aov_records): the wavefront kernels take an AovView by value, and one that holds nothing but
+// the planes keeps the parameters of the kernels of frames without planes as they are.
 struct AovView {
     McAovTargets planes;
+};
+
+// Per path, the camera ray's closest hit as the planes need it, written by k_wf_trace and folded per pixel by the
+// resolve kernels: distance and McHit-style id (-1: miss); for the guide planes also McHit.normal (xyz) and
+// McHit.tex_color, for hits only.  wavefront_carve puts them right after the queue counters, in this order, each
+// array 256-byte aligned.
+struct AovRecords {
     float* t;
     int* id;
+    float4* normal;
+    float4* albedo;
 };
+__host__ __device__ inline size_t aov_align256(size_t v) { return (v + 255) & ~static_cast<size_t>(255); }
+__host__ __device__ inline AovRecords aov_records(const WaveView& wv) {
+    unsigned char* const base = reinterpret_cast<unsigned char*>(wv.qCount) + 256;  // (the counters take 16 bytes)
+    const size_t cap = wv.pathCapacity;
+    AovRecords r;
+    r.t = reinterpret_cast<float*>(base);
+    r.id = reinterpret_cast<int*>(base + aov_align256(cap * sizeof(float)));
+    r.normal = reinterpret_cast<float4*>(base + 2 * aov_align256(cap * sizeof(float)));
+    r.albedo = r.normal + aov_align256(cap * sizeof(float4)) / sizeof(float4);
+    return r;
+}
 
 enum : int {
     kShadowHard = 0,      // no soft shadows: one ray to the light centre, normalised normal (shade())
@@ -86,19 +107,19 @@ struct BatchSlice {
 static_assert(sizeof(BatchSlice) == 256, "a BatchSlice is indexed by blockIdx.y: keep its stride a power of two");
 
 // Storage: per path (terminal colour, stack height, bounce stack), per queue entry (hit record + lit counter).
-// aov: the frame writes AOV planes (8 more bytes per path).
-size_t wavefront_bytes_per_path(const DevFrame& fr, bool aov = false);
+// aov: the frame writes AOV planes (8 more bytes per path); guides: normal or albedo among them (32 more).
+size_t wavefront_bytes_per_path(const DevFrame& fr, bool aov = false, bool guides = false);
 size_t wavefront_bytes_per_entry();
 size_t wavefront_fixed_bytes(const DevFrame& fr);
 // Hits a path can put into the queue: bounce levels + 1.  A queue of pathCapacity times this cannot overflow.
 int wavefront_max_hits_per_path(const DevFrame& fr);
 // Carves the views out of one allocation of at least pathCapacity * wavefront_bytes_per_path +
 // entryCapacity * wavefront_bytes_per_entry + wavefront_fixed_bytes (+ 256 per array) bytes; false if too small.
-// aov (frames with AOV planes): also carves its per-path records (aov->t, aov->id).
+// aov (frames with AOV planes): also carves the per-path records these planes need (aov_records).
 bool wavefront_carve(const DevFrame& fr, void* base, size_t bytes, unsigned int pathCapacity, unsigned int entryCapacity,
-                     int gridBlocks, WaveView* out, AovView* aov = nullptr);
+                     int gridBlocks, WaveView* out, const McAovTargets* aov = nullptr);
 
-// The AOV defaults (coverage 0, depth 0, tri_id -1) into every pixel of the band's tiles (of every scene of a batch), before
+// The AOV defaults (coverage 0, depth 0, tri_id -1, normal and albedo zeros) into every pixel of the band's tiles (of every scene of a batch), before
 // the primary pass; the shading pass then overwrites the pixels it resolves.  Only for bands with AOV planes.
 // aovBatch: the device array of a batch's per-scene AOV views (null: one frame, `planes`).
 void launch_aov_defaults(const DevFrame& fr, const BandView& band, const McAovTargets& planes, const AovView* aovBatch, int nScenes,

@@ -207,9 +207,10 @@ def render(scene, cfg: McConfig, device: int = 0, want_f32: bool = True, want_u8
     return f32, u8, {k: getattr(stats, k) for k, _ in McRenderStats._fields_}
 
 
-def render_aovs(scene, cfg: McConfig, device: int = 0, want_u8: bool = False):
+def render_aovs(scene, cfg: McConfig, device: int = 0, want_u8: bool = False, guides: bool = False):
     """mcskin_cuda_render_aovs: the frame of `render` plus its AOV planes.  Returns (f32 [H, W, 4], u8 [H, W, 4] | None,
-    {"coverage": float32 [H, W], "depth": float32 [H, W], "tri_id": int32 [H, W]}, stats dict)."""
+    {"coverage": float32 [H, W], "depth": float32 [H, W], "tri_id": int32 [H, W]}, stats dict).  guides: the planes also
+    hold "normal" float32 [H, W, 3] and "albedo" float32 [H, W, 4]."""
     h, w = max(cfg.height, 0), max(cfg.width, 0)
     f32 = np.empty((h, w, 4), dtype=np.float32)
     u8 = np.empty((h, w, 4), dtype=np.uint8) if want_u8 else None
@@ -222,7 +223,10 @@ def render_aovs(scene, cfg: McConfig, device: int = 0, want_u8: bool = False):
             u8[..., 3] = 255
     planes = {"coverage": np.empty((h, w), dtype=np.float32), "depth": np.empty((h, w), dtype=np.float32),
               "tri_id": np.empty((h, w), dtype=np.int32)}
-    targets = _abi.McAovTargets(planes["coverage"].ctypes.data, planes["depth"].ctypes.data, planes["tri_id"].ctypes.data)
+    if guides:
+        planes["normal"] = np.empty((h, w, 3), dtype=np.float32)
+        planes["albedo"] = np.empty((h, w, 4), dtype=np.float32)
+    targets = _abi.McAovTargets(*(planes[p].ctypes.data for p in planes))
     stats = McRenderStats()
     cs = scene.as_c() if isinstance(scene, FlatScene) else scene
     _check(_lib.mcskin_cuda_render_aovs(C.byref(cs), C.byref(cfg), C.c_int32(device), _ptr(f32, C.c_float),
@@ -355,10 +359,11 @@ class Context:
     def set_option(self, name: str, value: int):
         _check(_lib.mcskin_cuda_context_set_option(self._h, name.encode(), C.c_int64(value)))
 
-    def set_aov_targets(self, coverage: int = 0, depth: int = 0, tri_id: int = 0):
+    def set_aov_targets(self, coverage: int = 0, depth: int = 0, tri_id: int = 0, normal: int = 0, albedo: int = 0):
         """AOV planes for the following render calls: raw device addresses of float32 / float32 / int32 planes laid out
-        like the colour image of each call (0: that plane is not written; all 0 switches them off)."""
-        t = _abi.McAovTargets(coverage or None, depth or None, tri_id or None)
+        like the colour image of each call, and of float32 planes of 3 (normal) and 4 (albedo) values per pixel
+        (0: that plane is not written; all 0 switches them off)."""
+        t = _abi.McAovTargets(coverage or None, depth or None, tri_id or None, normal or None, albedo or None)
         _check(_lib.mcskin_cuda_context_set_aov_targets(self._h, C.byref(t)))
 
     def set_scene(self, scene: FlatScene, cfg: McConfig):
