@@ -1390,6 +1390,16 @@ static bool pix_kernel_applies(const DevFrame& fr, unsigned int blobBytes) {
     return need <= pix_smem_limit();
 }
 
+// The other kernels that stage the scene blob in dynamic shared memory keep static shared memory of their own
+// (k_primary_warp ~30 KB, k_primary_cta ~20 KB, k_shade_warp ~9 KB): with a blob near kMaxSceneSmemBytes their total
+// passes the default 48 KB and the launch is refused unless the kernel opted in (see SmemOptIn).
+static void blob_kernels_opt_in() {
+    static SmemOptIn optIn;
+    static const void* const fns[] = {reinterpret_cast<const void*>(k_primary_cta), reinterpret_cast<const void*>(k_primary_warp),
+                                      reinterpret_cast<const void*>(k_shade_cta), reinterpret_cast<const void*>(k_shade_warp)};
+    optIn.limit(fns, static_cast<int>(sizeof(fns) / sizeof(fns[0])));
+}
+
 bool launch_primary(const DevFrame& fr, const FramePointers& fp, const BandView& band, const ActiveList& list,
                     int classify, uint32_t* tileStates, bool seedTiles, int primaryTargetBlocks, int heavyTargetTiles,
                     cudaStream_t stream) {
@@ -1401,7 +1411,9 @@ bool launch_primary(const DevFrame& fr, const FramePointers& fp, const BandView&
         launch_primary_pix(fr, fp, band, list, tileStates, seedTiles, primaryTargetBlocks, heavyTargetTiles, nullptr, 1,
                            fp.blob_bytes, stream);
         return fr.draws_per_sample > 0;
-    } else if (classify && lg >= 0) {
+    }
+    blob_kernels_opt_in();
+    if (classify && lg >= 0) {
         k_primary_warp<<<nTiles, kBlockThreads, fp.blob_bytes, stream>>>(fr, fp, band, list, lg);
     } else {
         k_primary_cta<<<nTiles, kBlockThreads, fp.blob_bytes, stream>>>(fr, fp, band, list, classify);
@@ -1424,6 +1436,7 @@ int launch_shade(const DevFrame& fr, const FramePointers& fp, const BandView& ba
                  const McAovTargets* aov) {
     if (gridBlocks <= 0) return 0;
     const int lg = log2_if_warp_spp(fr.spp);
+    blob_kernels_opt_in();
     if (variant == 2 && lg >= 0)
         k_shade_warp<<<gridBlocks, kBlockThreads, fp.blob_bytes, stream>>>(fr, fp, band, list, lg, groupCounter, firstSlot);
     else

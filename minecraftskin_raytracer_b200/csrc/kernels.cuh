@@ -13,7 +13,8 @@
 namespace mcskin {
 
 constexpr int kBlockThreads = 256;
-// scene blob staged per CTA; 40 KB keeps the default 48 KB dynamic+static shared memory limit (227 boxes)
+// scene blob staged per CTA (SceneBlobLayout: 212 boxes at most); with a kernel's own static shared memory it can pass
+// the default 48 KB, so every kernel that stages it opts in to more (SmemOptIn)
 constexpr unsigned int kMaxSceneSmemBytes = 40u * 1024u;
 
 // Dynamic shared memory above the default 48 KB is an opt-in that CUDA keeps per function AND per

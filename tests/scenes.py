@@ -26,6 +26,23 @@ RENDER_CASES = [
     ("spp64", 14, "64x64", None, dict(width=40, height=40, samples_per_pixel=64, max_bounces=2)),
     ("spp300", 15, "64x64", None, dict(width=24, height=24, samples_per_pixel=300, max_bounces=1)),
     ("many_shadow_samples", 10, "64x64", None, dict(width=48, height=48, samples_per_pixel=1, max_bounces=1, shadow_samples=64)),
+    # route cases: kernel forms and shading routes the cases above never select (kernels.cu launch_primary_pix,
+    # wavefront.cu shadow_mode_of, dev_shade.cuh ambient_occlusion)
+    # flat 16-spp pixel-per-lane form; 13 shadow samples = one full round of 8 and a partial one; the largest AO that
+    # still draws from a FreshStream (2 * 113 <= 227)
+    ("flat16_sh13_ao113", 16, "64x64", "walking", dict(width=48, height=48, samples_per_pixel=16, max_bounces=2,
+                                                        gradient_bg=0, shadow_samples=13, ao_enabled=1, ao_samples=113)),
+    # flat 4-spp form; 114 shadow samples shade in-thread from a LocalEngine, 114 AO samples take ambient_occlusion_large
+    ("flat4_sh114_ao114", 17, "64x64", "dab", dict(width=48, height=48, samples_per_pixel=4, max_bounces=1, gradient_bg=0,
+                                                   tile_size=16, shadow_samples=114, ao_enabled=1, ao_samples=114)),
+    # generic pixel-per-lane form at spp x draws = 60, the largest ring that fits; one shadow sample: hard shadows
+    ("spp30_sh1", 18, "legacy", "running", dict(width=48, height=48, samples_per_pixel=30, max_bounces=2, shadow_samples=1)),
+    # generic form with lens draws at spp x draws = 60
+    ("dof_spp15", 19, "64x64", "fighting", dict(width=48, height=48, samples_per_pixel=15, max_bounces=1, dof_enabled=1,
+                                                aperture=0.4, shadow_samples=113)),
+    # lens draws at spp x draws = 64 > 61: the warp-per-pixel form
+    ("dof_spp16", 20, "64x64", None, dict(width=48, height=48, samples_per_pixel=16, max_bounces=2, dof_enabled=1,
+                                          aperture=0.3)),
 ]
 
 
