@@ -162,7 +162,11 @@ void mcskin_cuda_abi_sizes(int32_t* out8);
  * shading pass still runs.
  * out_rgba_f32 : width*height*4 floats (Image::pixels), may be NULL
  * out_rgba_u8  : width*height*4 bytes, uint8(clamp(c)*255+0.5) (image_writer.cpp:18-22), may be NULL
- * Renders on the current thread's CUDA device `device` (>= 0). */
+ * Renders on the current thread's CUDA device `device` (>= 0).
+ * Some configurations make NaN channels in the reference (ao_samples == 0 with AO on: 0/0 in computeAO; a negative
+ * shininess: inf*0 in shade()).  They are stored as x86's default NaN 0xffc00000, the bits the reference writes, here
+ * and in the float outputs of the single-query calls below (trace, shade, ambient_occlusion); their 8-bit value is 0.
+ * NaN payloads carried in by the inputs (NaN texels or config values) are not reproduced. */
 int32_t mcskin_cuda_render(const McScene* scene, const McConfig* cfg, int32_t device,
                            float* out_rgba_f32, uint8_t* out_rgba_u8,
                            McProgressFn progress, void* user, McRenderStats* stats);

@@ -57,6 +57,16 @@ __device__ __forceinline__ uint32_t seed_cast(float f) {
     return static_cast<uint32_t>(static_cast<unsigned long long>(__float2ll_rz(f)));
 }
 
+// A colour channel as the reference stores it.  With finite inputs every NaN the reference makes comes from its own
+// arithmetic (0.0f / 0.0f in computeAO with no samples, ks * inf * 0 in shade() with a negative shininess), where x86
+// gives the default NaN 0xffc00000 and each later operation passes it on unchanged; NVIDIA GPUs give 0x7fffffff.  So a
+// NaN leaves the device as 0xffc00000.  NaN payloads carried in by the inputs (NaN texels or config values) are not
+// reproduced.
+__device__ __forceinline__ float x86_nan(float c) { return c == c ? c : __uint_as_float(0xffc00000u); }
+__device__ __forceinline__ float4 x86_nan4(float4 c) {
+    return make_float4(x86_nan(c.x), x86_nan(c.y), x86_nan(c.z), x86_nan(c.w));
+}
+
 // uint8(clamp(c)*255 + 0.5) (image_writer.cpp:18-22)
 __device__ __forceinline__ uint32_t quantize8(float c) {
     return static_cast<uint32_t>(__float2int_rz(clamp01(c) * 255.0f + 0.5f)) & 0xffu;

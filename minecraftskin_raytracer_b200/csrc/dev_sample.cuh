@@ -64,6 +64,13 @@ __device__ __forceinline__ void store_pixel(const BandView& band, unsigned int i
     if (band.out_f32) band.out_f32[index] = c;
     if (band.out_u8) band.out_u8[index] = quantize4(c);
 }
+// A pixel with a shaded sample: a NaN channel leaves with the reference's bits (x86_nan).  A pixel whose samples all
+// missed is an average of background colours, which is never NaN when the background fields are finite, and is stored
+// as it is: the primary pass stores most pixels of a frame, and the check there cost the headline frame about 0.5 us
+// of its 754 (B200 at its 1000 W limit).
+__device__ __forceinline__ void store_shaded_pixel(const BandView& band, unsigned int index, float4 c) {
+    store_pixel(band, index, x86_nan4(c));
+}
 
 // The AOV planes of a pixel (McAovTargets), folded over its samples' camera-ray hits (the query whose miss gives a
 // sample the gradient, tile_renderer.cpp:111) in sample order: hit count, left-to-right sum of the hit distances,
@@ -130,16 +137,18 @@ constexpr int kWarpStageFloats = 32 * 4 + 32 * 4;
 // lane l carries sample l's colour.  Channel c of pixel p is summed IN SAMPLE ORDER by lane
 // 4p+c (so 4*32/spp lanes run the dependent add chains side by side), scaled by 1/spp and
 // written out.  resolveMask: bit p set = pixel p is resolved here; outIndex: the band-image
-// index held by the first lane of each pixel.
+// index held by the first lane of each pixel.  SHADED: the pixels hold shaded samples (see store_shaded_pixel).
 // outStage != null: the averages are not written to the image but to outStage[p] (p = pixel of the warp), for a caller
 // that collects the pixels of several calls and stores them together (the wavefront resolve: whole runs of
 // neighbouring pixels per store instead of 16 bytes at a time — the image may lie across PCIe or NVLink).
+template <bool SHADED>
 __device__ __forceinline__ void warp_resolve(const DevFrame& fr, const BandView& band, float* stageW, int lane,
                                              int spp, int lgSpp, float4 colour, unsigned int outIndex,
                                              unsigned int resolveMask, float4* outStage = nullptr) {
     if (spp == 1) {  // nothing to add: every lane writes its own pixel
         if ((resolveMask >> lane) & 1u) {
-            const float4 c = scale4(add4(make_float4(0.f, 0.f, 0.f, 0.f), colour), fr.inv_spp);
+            float4 c = scale4(add4(make_float4(0.f, 0.f, 0.f, 0.f), colour), fr.inv_spp);
+            if (SHADED) c = x86_nan4(c);
             if (outStage) outStage[lane] = c;
             else store_pixel(band, outIndex, c);
         }
@@ -160,6 +169,7 @@ __device__ __forceinline__ void warp_resolve(const DevFrame& fr, const BandView&
             const float* src = stageW + (p << lgSpp) * 4 + p * 4 + ch;
             for (int i = 0; i < spp; ++i) acc += src[i * 4];
             acc *= fr.inv_spp;
+            if (SHADED) acc = x86_nan(acc);  // (the image store below does not go through store_pixel)
         }
         if (outStage) {
             const float a1 = __shfl_down_sync(kFullMask, acc, 1);

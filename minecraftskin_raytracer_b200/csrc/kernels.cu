@@ -336,7 +336,7 @@ k_shade_cta(const DevFrame fr, const FramePointers fp, const BandView band, cons
             }
             __syncthreads();
         }
-        if (sumSp.x != kUnusedSlot) store_pixel(out, sumSp.x, scale4(acc, fr.inv_spp));
+        if (sumSp.x != kUnusedSlot) store_shaded_pixel(out, sumSp.x, scale4(acc, fr.inv_spp));
     }
 }
 
@@ -490,7 +490,7 @@ k_primary_warp(const DevFrame fr, const FramePointers fp, const BandView band, c
                 }
             }
             (void)validMask;
-            warp_resolve(fr, out, stageW, lane, spp, lgSpp, colour, outIndex, resolveMask);
+            warp_resolve<false>(fr, out, stageW, lane, spp, lgSpp, colour, outIndex, resolveMask);
 
             // work-list slots for the pixels with a hit: one atomic per warp
             const unsigned int leadersActive = __ballot_sync(kFullMask, leader && pixelActive);
@@ -1052,7 +1052,7 @@ k_shade_warp(const DevFrame fr, const FramePointers fp, const BandView band, con
                 resolveMask |= 1u << (l >> lgSpp);
             }
         }
-        warp_resolve(fr, out, stageW, lane, spp, lgSpp, colour, sp.x, resolveMask);
+        warp_resolve<true>(fr, out, stageW, lane, spp, lgSpp, colour, sp.x, resolveMask);
     }
 }
 
@@ -1157,7 +1157,7 @@ __global__ void k_trace(const DevFrame fr, const FramePointers fp, int depth, co
     opt.start_depth = depth;
     opt.primary_uv = false;
     opt.u = opt.v = 0.5f;
-    out[i] = trace_path(sc, fr, r, opt);
+    out[i] = x86_nan4(trace_path(sc, fr, r, opt));
 }
 
 __global__ void k_shade_hits(const DevFrame fr, const FramePointers fp, const McHit* hits, const float* viewDirs,
@@ -1166,9 +1166,9 @@ __global__ void k_shade_hits(const DevFrame fr, const FramePointers fp, const Mc
     if (i >= n) return;
     const SceneView sc = scene_view(fp.blob, fp.texels, fr);
     const McHit h = hits[i];
-    out[i] = shade_hit(sc, fr, ld3(h.point), ld3(h.normal),
-                       make_float4(h.tex_color[0], h.tex_color[1], h.tex_color[2], h.tex_color[3]),
-                       ld3(viewDirs + 3 * i), shadowFactors ? shadowFactors[i] : -1.0f);
+    out[i] = x86_nan4(shade_hit(sc, fr, ld3(h.point), ld3(h.normal),
+                                make_float4(h.tex_color[0], h.tex_color[1], h.tex_color[2], h.tex_color[3]),
+                                ld3(viewDirs + 3 * i), shadowFactors ? shadowFactors[i] : -1.0f));
 }
 
 __global__ void k_in_shadow(const DevFrame fr, const FramePointers fp, const float* points, const float* normals,
@@ -1193,7 +1193,7 @@ __global__ void k_ambient_occlusion(const DevFrame fr, const FramePointers fp, c
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const SceneView sc = scene_view(fp.blob, fp.texels, fr);
-    out[i] = ambient_occlusion(sc, ld3(points + 3 * i), ld3(normals + 3 * i), samples, radius, seeds[i]);
+    out[i] = x86_nan(ambient_occlusion(sc, ld3(points + 3 * i), ld3(normals + 3 * i), samples, radius, seeds[i]));
 }
 
 __global__ void k_generate_rays(const DevFrame fr, const float* uv, int n, McRay* out) {

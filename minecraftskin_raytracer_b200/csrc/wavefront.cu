@@ -526,7 +526,7 @@ k_wf_resolve_warp(const DevFrame fr, const BandView band_, const ActiveList list
             m &= m - 1u;
             resolveMask |= 1u << (l >> lgSpp);
         }
-        warp_resolve(fr, band, stageW, lane, spp, lgSpp, colour, pixelIndex, resolveMask, outStage);
+        warp_resolve<true>(fr, band, stageW, lane, spp, lgSpp, colour, pixelIndex, resolveMask, outStage);
         if (AOV && on && s == 0) {
             const AovView& av = BATCH ? aovBatch[blockIdx.y] : aov_;
             fold_aov(fr, av.planes, aov_records(wv), static_cast<size_t>(slot) * spp, spp, pixelIndex);
@@ -562,7 +562,7 @@ k_wf_resolve_warp(const DevFrame fr, const BandView band_, const ActiveList list
             round(base + local, pixelIndex, outW + g * pixPerGroup);
         }
         __syncwarp();
-        if (myPixel != kUnusedSlot) store_pixel(band, myPixel, outW[lane]);
+        if (myPixel != kUnusedSlot) store_pixel(band, myPixel, outW[lane]);  // (outW: warp_resolve<true> output)
         __syncwarp();
     }
 }
@@ -585,7 +585,7 @@ k_wf_resolve_pixel(const DevFrame fr, const BandView band_, const ActiveList lis
         if (sp.x == kUnusedSlot) continue;
         float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
         for (int s = 0; s < spp; ++s) acc = add4(acc, fold_path(wv, static_cast<size_t>(slot) * spp + s));
-        store_pixel(band, sp.x, scale4(acc, fr.inv_spp));
+        store_shaded_pixel(band, sp.x, scale4(acc, fr.inv_spp));
         if (AOV) {
             const AovView& av = BATCH ? aovBatch[blockIdx.y] : aov_;
             fold_aov(fr, av.planes, aov_records(wv), static_cast<size_t>(slot) * spp, spp, sp.x);
