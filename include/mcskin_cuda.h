@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define MCSKIN_ABI_VERSION 3
+#define MCSKIN_ABI_VERSION 4
 
 enum {
     MC_OK = 0,
@@ -189,18 +189,26 @@ int32_t mcskin_cuda_render(const McScene* scene, const McConfig* cfg, int32_t de
  * A hit never has a texel of alpha 0: such texels are passed through, and the outer-layer exit face is taken only when
  * its alpha is > 0.  So when no texel alpha is negative (every skin built from an 8-bit atlas), albedo's alpha is > 0
  * exactly where tri_id >= 0.
- * (normal and albedo were appended in ABI version 3.) */
+ * The skin-texel plane, one int32 per pixel: which texel of the scene's texture the pixel shows.
+ *   texel    : the texel index the first hitting sample's closest hit took (the sample tri_id reports), into
+ *              scene.texels_rgba: texels_rgba[4*texel .. 4*texel+3] == McHit.tex_color of that hit (for an outer-layer
+ *              hit that fell through to the exit face, the exit face's texel).  A face without texels gives the index
+ *              of a synthetic texel just past the pool: n_texels for a null texture (McFaceTex.texel_offset < 0,
+ *              magenta) and n_texels + 1 for an empty region (width <= 0 or height <= 0, (0, 0, 0, 1)).  -1 when n == 0,
+ *              so texel >= 0 exactly where tri_id >= 0.  In image i of a batch it indexes scene i's texels.
+ * (normal and albedo were appended in ABI version 3, texel in ABI version 4.) */
 typedef struct McAovTargets {
     float* coverage;
     float* depth;
     int32_t* tri_id;
     float* normal;
     float* albedo;
+    int32_t* texel;
 } McAovTargets;
 
 /* mcskin_cuda_render with AOV planes: the same colour bytes, and the planes `aov` asks for (host memory, width*height
  * values each, 3 and 4 times that for normal and albedo; aov may be NULL).  A frame with no tiles leaves the defaults
- * (0, 0, -1, zeros, zeros) in every requested plane. */
+ * (0, 0, -1, zeros, zeros, -1) in every requested plane. */
 int32_t mcskin_cuda_render_aovs(const McScene* scene, const McConfig* cfg, int32_t device,
                                 float* out_rgba_f32, uint8_t* out_rgba_u8, const McAovTargets* aov,
                                 McRenderStats* stats);

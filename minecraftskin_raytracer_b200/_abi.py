@@ -9,7 +9,7 @@ import ctypes as C
 
 import numpy as np
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 MC_OK = 0
 MC_ERR_INVALID = -1
@@ -101,7 +101,7 @@ class McRenderStats(C.Structure):
 class McAovTargets(C.Structure):
     """Per-pixel planes rendered next to the colour (include/mcskin_cuda.h); null members are not written."""
     _fields_ = [("coverage", C.c_void_p), ("depth", C.c_void_p), ("tri_id", C.c_void_p), ("normal", C.c_void_p),
-                ("albedo", C.c_void_p)]
+                ("albedo", C.c_void_p), ("texel", C.c_void_p)]
 
 
 class McRay(C.Structure):

@@ -155,7 +155,7 @@ struct McContext : McOptions {
         int nTiles, nHeavy;
         const void *hotF32, *hotU8;
         const void *aovCoverage, *aovDepth, *aovTriId;  // a graph with AOV stores is never replayed without them, or vice versa
-        const void *aovNormal, *aovAlbedo;
+        const void *aovNormal, *aovAlbedo, *aovTexel;
         long long optionBits[kOptionCount];             // the launch options (0 for the others)
         unsigned long long allocEpoch;
         bool operator==(const GraphKey& o) const { return std::memcmp(this, &o, sizeof(GraphKey)) == 0; }
@@ -219,6 +219,7 @@ inline McAovTargets aov_at(const McAovTargets& a, size_t pixels) {
     r.tri_id = a.tri_id ? a.tri_id + pixels : nullptr;
     r.normal = a.normal ? a.normal + 3 * pixels : nullptr;
     r.albedo = a.albedo ? a.albedo + 4 * pixels : nullptr;
+    r.texel = a.texel ? a.texel + pixels : nullptr;
     return r;
 }
 

@@ -119,6 +119,11 @@ __device__ __forceinline__ void store_guides(const McAovTargets& planes, unsigne
         o[3] = n > 0 ? f.a / fn : 0.0f;
     }
 }
+// The texel plane of a pixel (McAovTargets::texel): Hit::texel of its first hitting sample, the one whose id the AovFold
+// keeps; -1 when no sample hits.
+__device__ __forceinline__ void store_texel(const McAovTargets& planes, unsigned int index, int texel) {
+    if (planes.texel) planes.texel[index] = texel;
+}
 
 __device__ __forceinline__ float4 add4(float4 a, float4 b) {
     return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);

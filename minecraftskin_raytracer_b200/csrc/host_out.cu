@@ -332,6 +332,7 @@ int32_t mcskin_cuda_render_aovs(const McScene* scene, const McConfig* cfg, int32
         if (want.tri_id) std::fill(want.tri_id, want.tri_id + pixels, -1);
         if (want.normal) std::fill(want.normal, want.normal + 3 * pixels, 0.0f);
         if (want.albedo) std::fill(want.albedo, want.albedo + 4 * pixels, 0.0f);
+        if (want.texel) std::fill(want.texel, want.texel + pixels, -1);
         if (stats) *stats = McRenderStats{};
         return MC_OK;
     }
@@ -340,7 +341,7 @@ int32_t mcskin_cuda_render_aovs(const McScene* scene, const McConfig* cfg, int32
     int rc = shared_context(device, &ctx);
     if (rc != MC_OK) return rc;
     CU_TRY(cudaSetDevice(ctx->device));
-    CU_TRY(ctx->aovPlanes.reserve(std::max<size_t>(16, pixels * 10 * sizeof(float))));  // 1 + 1 + 1 + 3 + 4 values a pixel
+    CU_TRY(ctx->aovPlanes.reserve(std::max<size_t>(16, pixels * 11 * sizeof(float))));  // 1 + 1 + 1 + 3 + 4 + 1 values a pixel
     float* const base = static_cast<float*>(ctx->aovPlanes.p);
     McAovTargets dev{};
     dev.coverage = want.coverage ? base : nullptr;
@@ -348,6 +349,7 @@ int32_t mcskin_cuda_render_aovs(const McScene* scene, const McConfig* cfg, int32
     dev.tri_id = want.tri_id ? reinterpret_cast<int32_t*>(base + 2 * pixels) : nullptr;
     dev.normal = want.normal ? base + 3 * pixels : nullptr;
     dev.albedo = want.albedo ? base + 6 * pixels : nullptr;
+    dev.texel = want.texel ? reinterpret_cast<int32_t*>(base + 10 * pixels) : nullptr;
     ctx->aov = dev;
     rc = render_host(ctx, scene, cfg, outF32, outU8, stats);
     ctx->aov = McAovTargets{};
@@ -358,6 +360,7 @@ int32_t mcskin_cuda_render_aovs(const McScene* scene, const McConfig* cfg, int32
     if (want.tri_id) CU_TRY(cudaMemcpyAsync(want.tri_id, dev.tri_id, pixels * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
     if (want.normal) CU_TRY(cudaMemcpyAsync(want.normal, dev.normal, 3 * pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     if (want.albedo) CU_TRY(cudaMemcpyAsync(want.albedo, dev.albedo, 4 * pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    if (want.texel) CU_TRY(cudaMemcpyAsync(want.texel, dev.texel, pixels * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
     CU_TRY(cudaStreamSynchronize(ctx->stream));
     return MC_OK;
 }

@@ -1069,6 +1069,7 @@ k_aov_defaults(const DevFrame fr, const BandView band, const McAovTargets planes
         const unsigned int index = static_cast<unsigned int>(tg.bandRow0 + ly) * static_cast<unsigned int>(fr.width) + (tg.x + lx);
         store_aov(fr, planes, index, AovFold{});
         store_guides(planes, index, 0, GuideFold{});
+        store_texel(planes, index, -1);
     }
 }
 
@@ -1089,6 +1090,7 @@ k_aov_listed(const DevFrame fr, const FramePointers fp, const ActiveList list, c
         const int px = static_cast<int>(sp.y & 0xffffu), py = static_cast<int>(sp.y >> 16);
         AovFold a;
         GuideFold g;
+        int texel = -1;
         for (int s = 0; s < spp; ++s) {
             float d0 = 0.0f, d1 = 0.0f, d2 = 0.0f, d3 = 0.0f;
             const float* rec = list.records + (static_cast<size_t>(slot) * spp + s) * dps;
@@ -1103,6 +1105,7 @@ k_aov_listed(const DevFrame fr, const FramePointers fp, const ActiveList list, c
             float u, v;
             sample_uv(fr, px, py, sd, &u, &v);
             const Hit h = closest_hit(sc, primary_ray(fr, u, v, sd));
+            if (a.n == 0 && h.box >= 0) texel = h.texel;
             a.add(h.t, aov_id(h));
             if (guides && h.box >= 0) {
                 const V3 n = hit_normal(sc, h);
@@ -1110,6 +1113,7 @@ k_aov_listed(const DevFrame fr, const FramePointers fp, const ActiveList list, c
             }
         }
         store_aov(fr, planes, sp.x, a);
+        store_texel(planes, sp.x, texel);
         if (guides) store_guides(planes, sp.x, a.n, g);
     }
 }

@@ -94,7 +94,7 @@ __host__ __device__ inline int band_tile_count(const BandView& band, int tilesX)
 // AOV instantiations of the shading kernels when any plane is set, and the kernels of frames without run as before.
 // (Not members of BandView: the batched primary kernels copy a scene's BandView, and a larger one costs them registers.)
 __host__ __device__ inline bool aov_any(const McAovTargets* a) {
-    return a && (a->coverage || a->depth || a->tri_id || a->normal || a->albedo);
+    return a && (a->coverage || a->depth || a->tri_id || a->normal || a->albedo || a->texel);
 }
 // the guide planes (normal, albedo): they need the camera ray's normal and texel colour as well as its distance and id
 __host__ __device__ inline bool aov_guides(const McAovTargets& a) { return a.normal || a.albedo; }

@@ -85,7 +85,7 @@ __device__ __forceinline__ bool enqueue_hit(const HitQueueView& q, unsigned int*
 constexpr int kPathOverflow = -2;  // top[path]: the queue was full; the path is redone in-thread (k_wf_overflow)
 
 // AOV: also record every path's camera-ray hit for the AOV planes (aov_records; the normal and texel colour only when the
-// frame has a guide plane).
+// frame has a guide plane, the texel index only when it has the texel plane).
 template <bool BATCH, bool AOV>
 __global__ void WF_HIT0_BOUNDS
 k_wf_trace(const DevFrame fr, const FramePointers fp_, const ActiveList list_, const WaveView wv_, const AovView aov_,
@@ -139,7 +139,7 @@ k_wf_trace(const DevFrame fr, const FramePointers fp_, const ActiveList list_, c
                 hit = closest_hit(sc, ray);
                 if (AOV) {
                     const AovView& av = BATCH ? aovBatch[blockIdx.y] : aov_;
-                    const AovRecords rec = aov_records(wv);
+                    const AovRecords rec = aov_records(wv, av.planes);
                     rec.t[p] = hit.t;
                     rec.id[p] = aov_id(hit);
                     if (aov_guides(av.planes) && hit.box >= 0) {
@@ -147,6 +147,7 @@ k_wf_trace(const DevFrame fr, const FramePointers fp_, const ActiveList list_, c
                         rec.normal[p] = make_float4(n.x, n.y, n.z, 0.0f);
                         rec.albedo[p] = hit_texel(sc, hit);
                     }
+                    if (av.planes.texel) rec.texel[p] = hit.texel;
                 }
                 if (fr.max_bounces < 0) {
                     // traceRay returns at once (depth 0 > maxBounces, raytracer.cpp:86-90); the tile
@@ -482,6 +483,15 @@ __device__ __forceinline__ void fold_aov(const DevFrame& fr, const McAovTargets&
     AovFold a;
     for (int i = 0; i < spp; ++i) a.add(rec.t[path0 + i], rec.id[path0 + i]);
     store_aov(fr, planes, pixelIndex, a);
+    if (planes.texel) {
+        int texel = -1;
+        for (int i = 0; i < spp; ++i)
+            if (rec.id[path0 + i] >= 0) {
+                texel = rec.texel[path0 + i];
+                break;
+            }
+        store_texel(planes, pixelIndex, texel);
+    }
     if (!aov_guides(planes)) return;
     GuideFold g;
     for (int i = 0; i < spp; ++i)
@@ -492,7 +502,7 @@ __device__ __forceinline__ void fold_aov(const DevFrame& fr, const McAovTargets&
 // FAR: the form for images across a link (BandView::far_output); two instantiations, so that the streaming form keeps
 // its 32 registers (8 resident blocks: the kernel lives on loads in flight).
 // AOV: the first lane of every pixel also folds the pixel's recorded camera-ray hits in sample order (store_aov,
-// store_guides).
+// store_texel, store_guides).
 template <bool BATCH, bool FAR, bool AOV>
 __global__ void __launch_bounds__(kWfThreads)
 k_wf_resolve_warp(const DevFrame fr, const BandView band_, const ActiveList list_, const WaveView wv_, const int lgSpp,
@@ -529,7 +539,7 @@ k_wf_resolve_warp(const DevFrame fr, const BandView band_, const ActiveList list
         warp_resolve<true>(fr, band, stageW, lane, spp, lgSpp, colour, pixelIndex, resolveMask, outStage);
         if (AOV && on && s == 0) {
             const AovView& av = BATCH ? aovBatch[blockIdx.y] : aov_;
-            fold_aov(fr, av.planes, aov_records(wv), static_cast<size_t>(slot) * spp, spp, pixelIndex);
+            fold_aov(fr, av.planes, aov_records(wv, av.planes), static_cast<size_t>(slot) * spp, spp, pixelIndex);
         }
     };
     if (!FAR) {
@@ -588,7 +598,7 @@ k_wf_resolve_pixel(const DevFrame fr, const BandView band_, const ActiveList lis
         store_shaded_pixel(band, sp.x, scale4(acc, fr.inv_spp));
         if (AOV) {
             const AovView& av = BATCH ? aovBatch[blockIdx.y] : aov_;
-            fold_aov(fr, av.planes, aov_records(wv), static_cast<size_t>(slot) * spp, spp, sp.x);
+            fold_aov(fr, av.planes, aov_records(wv, av.planes), static_cast<size_t>(slot) * spp, spp, sp.x);
         }
     }
 }
@@ -624,10 +634,10 @@ constexpr int kQueueCounters = 4;
 }  // namespace
 
 int wavefront_max_hits_per_path(const DevFrame& fr) { return stack_levels_of(fr) + 1; }
-size_t wavefront_bytes_per_path(const DevFrame& fr, bool aov, bool guides) {
-    // tail, top, bounce stack (+ the camera ray's hit distance and id, + its normal and texel colour)
+size_t wavefront_bytes_per_path(const DevFrame& fr, bool aov, bool guides, bool texel) {
+    // tail, top, bounce stack (+ the camera ray's hit distance and id, + its normal and texel colour, + its texel index)
     return sizeof(float4) + sizeof(int) + sizeof(float4) * stack_levels_of(fr) + (aov ? sizeof(float) + sizeof(int) : 0) +
-           (aov && guides ? 2 * sizeof(float4) : 0);
+           (aov && guides ? 2 * sizeof(float4) : 0) + (aov && texel ? sizeof(int) : 0);
 }
 size_t wavefront_bytes_per_entry() { return kEntryBytes; }
 size_t wavefront_fixed_bytes(const DevFrame&) { return 256 * 16 + sizeof(unsigned int) * kQueueCounters; }
@@ -661,12 +671,13 @@ bool wavefront_carve(const DevFrame& fr, void* base, size_t bytes, unsigned int 
     // [0] hits in the queue (counts on beyond the capacity: overflow), [1] chunk counter of the soft-shadow kernel
     w.qCount = static_cast<unsigned int*>(take(sizeof(unsigned int) * kQueueCounters));
     if (aov) {  // in aov_records' order, right after the counters
-        if (take(cap * sizeof(float)) != aov_records(w).t) return false;
+        if (take(cap * sizeof(float)) != aov_records(w, *aov).t) return false;
         take(cap * sizeof(int));
         if (aov_guides(*aov)) {
             take(cap * sizeof(float4));
             take(cap * sizeof(float4));
         }
+        if (aov->texel) take(cap * sizeof(int));
     }
     if (off > bytes) return false;
     *out = w;

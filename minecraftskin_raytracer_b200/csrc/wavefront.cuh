@@ -68,23 +68,26 @@ struct AovView {
 
 // Per path, the camera ray's closest hit as the planes need it, written by k_wf_trace and folded per pixel by the
 // resolve kernels: distance and McHit-style id (-1: miss); for the guide planes also McHit.normal (xyz) and
-// McHit.tex_color, for hits only.  wavefront_carve puts them right after the queue counters, in this order, each
-// array 256-byte aligned.
+// McHit.tex_color, for hits only; for the texel plane Hit::texel.  wavefront_carve puts them right after the queue
+// counters, in this order, each array 256-byte aligned; normal and albedo take no room in frames without guide planes.
 struct AovRecords {
     float* t;
     int* id;
     float4* normal;
     float4* albedo;
+    int* texel;
 };
 __host__ __device__ inline size_t aov_align256(size_t v) { return (v + 255) & ~static_cast<size_t>(255); }
-__host__ __device__ inline AovRecords aov_records(const WaveView& wv) {
+__host__ __device__ inline AovRecords aov_records(const WaveView& wv, const McAovTargets& planes) {
     unsigned char* const base = reinterpret_cast<unsigned char*>(wv.qCount) + 256;  // (the counters take 16 bytes)
     const size_t cap = wv.pathCapacity;
+    const size_t a4 = aov_align256(cap * sizeof(float)), a16 = aov_align256(cap * sizeof(float4));
     AovRecords r;
     r.t = reinterpret_cast<float*>(base);
-    r.id = reinterpret_cast<int*>(base + aov_align256(cap * sizeof(float)));
-    r.normal = reinterpret_cast<float4*>(base + 2 * aov_align256(cap * sizeof(float)));
-    r.albedo = r.normal + aov_align256(cap * sizeof(float4)) / sizeof(float4);
+    r.id = reinterpret_cast<int*>(base + a4);
+    r.normal = reinterpret_cast<float4*>(base + 2 * a4);
+    r.albedo = reinterpret_cast<float4*>(base + 2 * a4 + a16);
+    r.texel = reinterpret_cast<int*>(base + 2 * a4 + (aov_guides(planes) ? 2 * a16 : 0));
     return r;
 }
 
@@ -107,8 +110,9 @@ struct BatchSlice {
 static_assert(sizeof(BatchSlice) == 256, "a BatchSlice is indexed by blockIdx.y: keep its stride a power of two");
 
 // Storage: per path (terminal colour, stack height, bounce stack), per queue entry (hit record + lit counter).
-// aov: the frame writes AOV planes (8 more bytes per path); guides: normal or albedo among them (32 more).
-size_t wavefront_bytes_per_path(const DevFrame& fr, bool aov = false, bool guides = false);
+// aov: the frame writes AOV planes (8 more bytes per path); guides: normal or albedo among them (32 more); texel: the
+// texel plane among them (4 more).
+size_t wavefront_bytes_per_path(const DevFrame& fr, bool aov = false, bool guides = false, bool texel = false);
 size_t wavefront_bytes_per_entry();
 size_t wavefront_fixed_bytes(const DevFrame& fr);
 // Hits a path can put into the queue: bounce levels + 1.  A queue of pathCapacity times this cannot overflow.
@@ -119,7 +123,7 @@ int wavefront_max_hits_per_path(const DevFrame& fr);
 bool wavefront_carve(const DevFrame& fr, void* base, size_t bytes, unsigned int pathCapacity, unsigned int entryCapacity,
                      int gridBlocks, WaveView* out, const McAovTargets* aov = nullptr);
 
-// The AOV defaults (coverage 0, depth 0, tri_id -1, normal and albedo zeros) into every pixel of the band's tiles (of every scene of a batch), before
+// The AOV defaults (coverage 0, depth 0, tri_id -1, normal and albedo zeros, texel -1) into every pixel of the band's tiles (of every scene of a batch), before
 // the primary pass; the shading pass then overwrites the pixels it resolves.  Only for bands with AOV planes.
 // aovBatch: the device array of a batch's per-scene AOV views (null: one frame, `planes`).
 void launch_aov_defaults(const DevFrame& fr, const BandView& band, const McAovTargets& planes, const AovView* aovBatch, int nScenes,

@@ -167,6 +167,28 @@ def skin_layout(atlas: np.ndarray, pose=None):
     return boxes[:cs.n_boxes].copy(), faces[:n_faces.value].copy(), opaque[:cs.n_boxes].copy(), int(cs.n_texels)
 
 
+def skin_texel_atlas(atlas: np.ndarray) -> np.ndarray:
+    """Atlas pixel of every texel of the skin's scene: int32 [n_texels + 2, 2] of (x, y), so that texel k of
+    build_skin_scene(atlas) is atlas[y, x] / 255.0f.  Built from skin_layout's face windows: the texel at (col, row) of a
+    window comes from (x + (w - 1 - col if mirror else col), y + row).
+
+    Index it with a texel plane (render_aovs(..., texel=True), Context.set_aov_targets(texel=...)): the last two rows,
+    the synthetic null-texture and empty-region texels, are (-1, -1), and so is the -1 of a pixel no sample hits,
+    because numpy reads index -1 as the last row.
+
+    The table depends on the atlas (an outer layer whose texels are all transparent is not built, and the texels of
+    the boxes after it move down the pool) but not on the pose: a pose turns boxes and leaves their texels alone."""
+    _, faces, _, n_texels = skin_layout(atlas)
+    table = np.full((n_texels + 2, 2), -1, dtype=np.int32)
+    for dst, x, y, w, h, mirror in faces:
+        col = np.arange(w, dtype=np.int32)
+        xs = x + (w - 1 - col if mirror else col)
+        ys = y + np.arange(h, dtype=np.int32)
+        table[dst:dst + w * h, 0] = np.tile(xs, h)
+        table[dst:dst + w * h, 1] = np.repeat(ys, w)
+    return table
+
+
 # ---------------------------------------------------------------- whole-frame calls
 def render(scene, cfg: McConfig, device: int = 0, want_f32: bool = True, want_u8: bool = False,
            progress=None, multi_devices: int = 0, out_f32: np.ndarray | None = None, out_u8: np.ndarray | None = None):
@@ -207,10 +229,11 @@ def render(scene, cfg: McConfig, device: int = 0, want_f32: bool = True, want_u8
     return f32, u8, {k: getattr(stats, k) for k, _ in McRenderStats._fields_}
 
 
-def render_aovs(scene, cfg: McConfig, device: int = 0, want_u8: bool = False, guides: bool = False):
+def render_aovs(scene, cfg: McConfig, device: int = 0, want_u8: bool = False, guides: bool = False, texel: bool = False):
     """mcskin_cuda_render_aovs: the frame of `render` plus its AOV planes.  Returns (f32 [H, W, 4], u8 [H, W, 4] | None,
     {"coverage": float32 [H, W], "depth": float32 [H, W], "tri_id": int32 [H, W]}, stats dict).  guides: the planes also
-    hold "normal" float32 [H, W, 3] and "albedo" float32 [H, W, 4]."""
+    hold "normal" float32 [H, W, 3] and "albedo" float32 [H, W, 4].  texel: they also hold "texel" int32 [H, W], the
+    texel index of the first hitting sample (-1: no hit; see skin_texel_atlas for a skin's atlas pixels)."""
     h, w = max(cfg.height, 0), max(cfg.width, 0)
     f32 = np.empty((h, w, 4), dtype=np.float32)
     u8 = np.empty((h, w, 4), dtype=np.uint8) if want_u8 else None
@@ -226,7 +249,9 @@ def render_aovs(scene, cfg: McConfig, device: int = 0, want_u8: bool = False, gu
     if guides:
         planes["normal"] = np.empty((h, w, 3), dtype=np.float32)
         planes["albedo"] = np.empty((h, w, 4), dtype=np.float32)
-    targets = _abi.McAovTargets(*(planes[p].ctypes.data for p in planes))
+    if texel:
+        planes["texel"] = np.empty((h, w), dtype=np.int32)
+    targets = _abi.McAovTargets(**{p: planes[p].ctypes.data for p in planes})
     stats = McRenderStats()
     cs = scene.as_c() if isinstance(scene, FlatScene) else scene
     _check(_lib.mcskin_cuda_render_aovs(C.byref(cs), C.byref(cfg), C.c_int32(device), _ptr(f32, C.c_float),
@@ -359,11 +384,13 @@ class Context:
     def set_option(self, name: str, value: int):
         _check(_lib.mcskin_cuda_context_set_option(self._h, name.encode(), C.c_int64(value)))
 
-    def set_aov_targets(self, coverage: int = 0, depth: int = 0, tri_id: int = 0, normal: int = 0, albedo: int = 0):
-        """AOV planes for the following render calls: raw device addresses of float32 / float32 / int32 planes laid out
-        like the colour image of each call, and of float32 planes of 3 (normal) and 4 (albedo) values per pixel
-        (0: that plane is not written; all 0 switches them off)."""
-        t = _abi.McAovTargets(coverage or None, depth or None, tri_id or None, normal or None, albedo or None)
+    def set_aov_targets(self, coverage: int = 0, depth: int = 0, tri_id: int = 0, normal: int = 0, albedo: int = 0,
+                        texel: int = 0):
+        """AOV planes for the following render calls: raw device addresses of float32 / float32 / int32 / int32 (texel)
+        planes laid out like the colour image of each call, and of float32 planes of 3 (normal) and 4 (albedo) values per
+        pixel (0: that plane is not written; all 0 switches them off)."""
+        t = _abi.McAovTargets(coverage or None, depth or None, tri_id or None, normal or None, albedo or None,
+                              texel or None)
         _check(_lib.mcskin_cuda_context_set_aov_targets(self._h, C.byref(t)))
 
     def set_scene(self, scene: FlatScene, cfg: McConfig):

@@ -1,7 +1,9 @@
-"""What the guide planes (normal, albedo; McAovTargets) cost on the GPU, next to the three planes before them.
+"""What the guide planes (normal, albedo) and the texel plane (McAovTargets) cost on the GPU, next to the three planes
+before them.
 
 The headline frame (bench.py's workload: 1920x1080, 16 spp, 4 bounces, one context, render_rows_into_frame into a
-device frame) with no planes, with coverage + depth + tri_id, and with all five planes, alternating in rounds: CUDA
+device frame) with no planes, with coverage + depth + tri_id, with the five planes up to albedo and with all six,
+alternating in rounds: CUDA
 events around every frame, a 256 MiB fill before each (outside the events) so that no frame finds the last one in L2,
 graph replay as in the bench.  Prints one JSON object (and writes it to --out): the card, its power limit, the numbers.
 
@@ -21,7 +23,7 @@ sys.dont_write_bytecode = True
 
 from tools.aov_bench import card  # noqa: E402
 
-FORMS = ("none", "three", "five")
+FORMS = ("none", "three", "five", "six")
 
 
 def main():
@@ -53,11 +55,12 @@ def main():
               "depth": torch.zeros((H, W), dtype=torch.float32, device=dev),
               "tri_id": torch.zeros((H, W), dtype=torch.int32, device=dev),
               "normal": torch.zeros((H, W, 3), dtype=torch.float32, device=dev),
-              "albedo": torch.zeros((H, W, 4), dtype=torch.float32, device=dev)}
+              "albedo": torch.zeros((H, W, 4), dtype=torch.float32, device=dev),
+              "texel": torch.zeros((H, W), dtype=torch.int32, device=dev)}
     ctx = {f: lib.Context(0) for f in FORMS}  # one context per form: each keeps its own captured graph
     for form, c in ctx.items():
         c.set_scene(scene, cfg)
-        names = {"none": (), "three": ("coverage", "depth", "tri_id"), "five": tuple(planes)}[form]
+        names = {"none": (), "three": ("coverage", "depth", "tri_id"), "five": tuple(planes)[:5], "six": tuple(planes)}[form]
         if names:
             c.set_aov_targets(**{p: planes[p].data_ptr() for p in names})
 
@@ -79,7 +82,7 @@ def main():
         frames(form, args.warmup, False)
     per = {f: [] for f in FORMS}
     for r in range(args.rounds):
-        order = FORMS[r % 3:] + FORMS[:r % 3]  # every form leads a round in turn
+        order = FORMS[r % len(FORMS):] + FORMS[:r % len(FORMS)]  # every form leads a round in turn
         for form in order:
             per[form].append(statistics.mean(frames(form, args.steps, True)))
     launches = {f: ctx[f].sync()["n_kernel_launches"] for f in FORMS}
@@ -91,14 +94,16 @@ def main():
         "card": card(),
         "headline_1080p_16spp_4b": {
             "ms_per_frame": med,
-            "overhead_pct_vs_none": {f: 100.0 * (med[f] - med["none"]) / med["none"] for f in ("three", "five")},
+            "round_spread_ms": {f: max(per[f]) - min(per[f]) for f in FORMS},
+            "overhead_pct_vs_none": {f: 100.0 * (med[f] - med["none"]) / med["none"] for f in FORMS[1:]},
             "overhead_pct_five_vs_three": 100.0 * (med["five"] - med["three"]) / med["three"],
+            "overhead_us_six_vs_five": 1000.0 * (med["six"] - med["five"]),
             "round_means": per,
             "kernel_launches_per_frame": launches,
-            "plane_bytes_stored_per_frame": {"three": H * W * 12, "five": H * W * 40},
+            "plane_bytes_stored_per_frame": {"three": H * W * 12, "five": H * W * 40, "six": H * W * 44},
             "what": f"{args.rounds} rounds of {args.steps} frames per form, the forms in rotating order, after {args.warmup} "
                     "warm-up frames each; CUDA events around each render_rows_into_frame (graph replay), 256 MiB L2 flush "
-                    "before each frame outside the events; median of the round means",
+                    "before each frame outside the events; median of the round means, spread = largest - smallest",
         },
     }
     text = json.dumps(out, indent=1)
