@@ -355,6 +355,32 @@ int32_t mcskin_cuda_context_render_skin_batch(McContext* ctx, const uint8_t* atl
 int32_t mcskin_cuda_render_batch_multi(const McScene* scenes, int32_t n_scenes, const McConfig* cfg, int32_t n_devices,
                                        float* out_rgba_f32, uint8_t* out_rgba_u8);
 
+/* ---- PNG files made on the device ----
+ * Every file is a valid PNG of one width x height 8-bit RGBA image (colour type 6, no interlace) holding only the
+ * chunks IHDR, IDAT (one or more) and IEND, each with its CRC-32.  Its bytes are fixed by the image alone:
+ *  - Row filters: each row takes the filter type (0 None .. 4 Paeth) whose filtered bytes, read as signed 8-bit
+ *    values, have the smallest sum of absolute values (libpng's heuristic); on a tie the lower type.
+ *  - Deflate: the filtered stream (per row its filter-type byte, then 4*width bytes) is cut into segments of
+ *    32768 bytes, the last one shorter, each compressed on its own: no match reaches before its segment's start.  A
+ *    segment is one block with dynamic Huffman codes of at most 15 bits (greedy LZ77 over a hash chain), or, when
+ *    that would take more bytes than the segment has, one stored block.  Every segment then ends byte-aligned with
+ *    an empty stored block (00 00 ff ff, pigz's sync-flush marker); the last segment's is the final block (BFINAL).
+ *  - Segment k is the data of IDAT chunk k; the zlib header (78 01) opens the first, the Adler-32 of the filtered
+ *    stream closes the last.
+ * The same image gives the same bytes on every run, alone or at any place in a batch of any size. */
+
+/* The largest file of a width x height image: every segment stored.  Host code, no device needed.  0 when width
+ * or height is outside 1..65535. */
+uint64_t mcskin_png_bound(int32_t width, int32_t height);
+/* PNG files of n_images consecutive width x height RGBA8 images in device memory (the u8 layout render_batch and
+ * render_skin_batch write), back to back into d_png (device, capacity bytes).  d_offsets (device, n_images + 1
+ * uint64) receives the exclusive prefix sums of the file sizes: file i is bytes [d_offsets[i], d_offsets[i+1]) and
+ * d_offsets[n_images] bytes in all, so one copy moves every file.  Asynchronous and ordered on `stream` (null: the
+ * context's); the scratch is the context's and grows with the images encoded together (up to about 1 GiB, at least
+ * one image).  MC_ERR_INVALID for a null pointer, a bad size or capacity < n_images * mcskin_png_bound. */
+int32_t mcskin_cuda_context_encode_png(McContext* ctx, const void* d_rgba8, int32_t width, int32_t height, int32_t n_images,
+                                       void* d_png, uint64_t capacity, uint64_t* d_offsets, void* stream);
+
 /* ---- single-ray entry points: the reference's free functions, exercised through
  *      the same device code (no CPU fallback).  All arrays are HOST memory. ---- */
 typedef struct McRay {

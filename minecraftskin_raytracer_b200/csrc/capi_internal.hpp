@@ -193,6 +193,7 @@ struct McContext : McOptions {
     // pointers, all null: none).  Child lanes get their parent's (inherit_options).
     McAovTargets aov{};
     DevBuf aovPlanes;                        // mcskin_cuda_render_aovs: the planes on the device before they go to the host
+    DevBuf pngScratch;                       // mcskin_cuda_context_encode_png: filtered streams, tokens, segments (png.cuh)
 };
 
 // The launchers of one of the three builds of the hot kernels (dev_types.cuh): the general form; no pose code, for

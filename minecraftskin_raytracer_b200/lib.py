@@ -41,6 +41,7 @@ EXPORTS = [
     "mcskin_cuda_enable_peer_access", "mcskin_cuda_context_render_scene_tiles",
     "mcskin_cuda_context_debug_block_times", "mcskin_cuda_context_render_skin_batch",
     "mcskin_skin_layout", "mcskin_cuda_render_aovs", "mcskin_cuda_context_set_aov_targets",
+    "mcskin_png_bound", "mcskin_cuda_context_encode_png",
 ]
 
 
@@ -68,6 +69,8 @@ def _load() -> C.CDLL:
     lib.mcskin_cuda_abi_sizes.restype = None
     lib.mcskin_counter_word.restype = C.c_uint32
     lib.mcskin_counter_word.argtypes = [C.c_uint32, C.c_uint32]
+    lib.mcskin_png_bound.restype = C.c_uint64
+    lib.mcskin_png_bound.argtypes = [C.c_int32, C.c_int32]
     return lib
 
 
@@ -124,6 +127,12 @@ def host_copy_rows(dst: np.ndarray, src: np.ndarray, row_bytes: int, rows: int, 
                                       C.c_uint64(row_bytes if dst_pitch is None else dst_pitch),
                                       C.c_uint64(row_bytes if src_pitch is None else src_pitch),
                                       C.c_uint64(row_bytes), C.c_uint64(rows), C.c_int32(pieces)))
+
+
+def png_bound(width: int, height: int) -> int:
+    """Bytes of the largest PNG file Context.encode_png makes of one width x height image (every segment stored);
+    0 when a side is outside 1..65535.  Host code."""
+    return int(_lib.mcskin_png_bound(width, height))
 
 
 def generate_tiles(width: int, height: int, tile_size: int) -> np.ndarray:
@@ -463,6 +472,35 @@ class Context:
                                                           C.c_void_p(d_out_f32 or None), C.c_void_p(d_out_u8 or None),
                                                           C.c_void_p(stream or None)))
         self.cfg = _abi.copy_config(cfg)
+
+    def encode_png(self, d_u8: int, width: int, height: int, n: int, d_png: int, capacity: int, d_offsets: int, stream: int = 0):
+        """Asynchronous: PNG files of the n [height, width, 4] uint8 device images at d_u8, back to back into d_png
+        (capacity >= n * png_bound(width, height) bytes); the n + 1 uint64 at d_offsets get the file offsets
+        (file i is bytes offsets[i]:offsets[i + 1]).  Addresses are raw device pointers."""
+        _check(_lib.mcskin_cuda_context_encode_png(self._h, C.c_void_p(d_u8 or None), C.c_int32(width), C.c_int32(height),
+                                                    C.c_int32(n), C.c_void_p(d_png or None), C.c_uint64(capacity),
+                                                    C.c_void_p(d_offsets or None), C.c_void_p(stream or None)))
+
+    def render_skin_batch_png(self, atlases: np.ndarray, cfg: McConfig, poses=None) -> list[bytes]:
+        """Blocking: render_skin_batch into a device uint8 buffer, encode_png, then one copy of all the files to the
+        host.  Returns the PNG file of every skin, in order."""
+        import torch
+        atlases = np.ascontiguousarray(atlases, dtype=np.uint8)
+        n = atlases.shape[0]
+        if n == 0:
+            return []
+        dev = torch.device("cuda", self.device)
+        stream = torch.cuda.Stream(dev)  # its own: torch's default stream does not order with the context's
+        with torch.cuda.stream(stream):
+            images = torch.empty((n, cfg.height, cfg.width, 4), dtype=torch.uint8, device=dev)
+            files = torch.empty(n * png_bound(cfg.width, cfg.height), dtype=torch.uint8, device=dev)
+            offsets = torch.empty(n + 1, dtype=torch.int64, device=dev)
+            self.render_skin_batch(atlases, cfg, poses, 0, images.data_ptr(), stream.cuda_stream)
+            self.encode_png(images.data_ptr(), cfg.width, cfg.height, n, files.data_ptr(), files.numel(), offsets.data_ptr(),
+                            stream.cuda_stream)
+            offs = offsets.cpu().tolist()  # (waits for the stream)
+            data = files[:offs[n]].cpu().numpy().tobytes()
+        return [data[offs[i]:offs[i + 1]] for i in range(n)]
 
     def debug_block_times(self) -> np.ndarray:
         """[n, 4] uint64 (entry ns, exit ns, frame tile, part | parts << 16) of the last primary launch
